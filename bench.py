@@ -4,6 +4,7 @@
     python bench.py --gpus N --steps K --warmup W            # this repo's CUDA path
     python bench.py --impl reference --gpus N --steps K ...  # the reference's CPU algorithm (oracle port)
     python bench.py --workload {train,beam4,beam8,lite,swin} # the other BASELINE.json configs (3, 4, 5), same contract
+    python bench.py ... --dump-outputs DIR                   # also save the last timed step's outputs as DIR/<name>.npy
 
 A "step" is one pass of the hot path (encode + 231-step greedy decode) over one
 synthetic batch of 256 images (128x256 grayscale, randn) per GPU.  `value` is
@@ -131,21 +132,49 @@ def synthetic_images(batch, seed):
     return torch.randn(batch, 1, 128, 256, generator=g)
 
 
+DUMP_BYTES = 60 * 10**6     # --dump-outputs stays under 64 MB with the .npy headers; the default greedy batch fits whole
+
+
+def dump_outputs(out_dir, arrays):
+    """Write each tensor as out_dir/<name>.npy: floating point as float32, integers (tokens) as float64, which holds them
+    exactly.  When they exceed DUMP_BYTES together, the same seeded subset of rows of the leading (batch) dimension is
+    kept of every array, so that two builds run with the same arguments still write comparable files."""
+    import numpy as np
+    arrs = {k: (v.float() if v.is_floating_point() else v.double()).cpu().numpy() for k, v in arrays.items()}
+    total = sum(a.nbytes for a in arrs.values())
+    if total > DUMP_BYTES:
+        n = next(iter(arrs.values())).shape[0]
+        keep = np.sort(np.random.default_rng(0).choice(n, max(1, n * DUMP_BYTES // total), replace=False))
+        arrs = {k: a[keep] for k, a in arrs.items()}
+    os.makedirs(out_dir, exist_ok=True)
+    for k, a in arrs.items():
+        np.save(os.path.join(out_dir, k + ".npy"), a)
+
+
 def workload_config(batch, precision):
     return {"workload": "EfficientSATRN greedy inference, batch %d per GPU, 128x256x1 randn images, "
-                        "max_sequence 230 (231 decode steps), random-init weights, image batch sharded "
+                        "max_sequence 230 (231 decode steps), seeded synthetic weights with calibrated BatchNorm "
+                        "statistics, image batch sharded "
                         "over ranks (no collective)" % batch,
             "batch_per_gpu": batch, "decode_steps": STEPS_PER_IMAGE, "precision": precision,
             "l2": "256 MiB buffer written between timed iterations (L2 flush); per-step working set "
                   "(KV cache + activations) also exceeds the 126 MB L2"}
 
 
+def checkpoint():
+    """The EfficientSATRN weights every EfficientSATRN workload runs: the seeded synthetic checkpoint of the parity
+    tests, whose BatchNorm running statistics are calibrated on a seeded batch.  With uncalibrated random-init
+    statistics the trunk's activations grow to ~1e7, beyond the fp16 range of the 16-bit encoder, and the 16-bit
+    workloads would time a pass whose logits are inf / NaN."""
+    from oracle import satrn, synth
+    return synth.synth_state_dict(satrn.ModelSpec(), 0)
+
+
 def build_model(precision, batch):
     import frx
     from helpers import Vocab, flags_dict
     flags = frx.Flags(flags_dict()).get()
-    dims = frx.layout.dims_from_flags(flags, 245)
-    sd = frx.synthetic.synthetic_state_dict(dims, seed=0)
+    sd = checkpoint()
     model = frx.EfficientSATRN(flags, Vocab(), sd, None, precision=precision, max_batch=batch,
                                max_steps=STEPS_PER_IMAGE)
     return model, sd
@@ -173,10 +202,7 @@ def run_reference(args, rank, world):
     if rank != 0:
         return
     import torch
-    import frx
-    from helpers import flags_dict
-    dims = frx.layout.dims_from_flags(frx.Flags(flags_dict()).get(), 245)
-    sd = frx.synthetic.synthetic_state_dict(dims, seed=0)
+    sd = checkpoint()
     if args.workload != "greedy":
         wl = args.workload
         if wl == "lite":
@@ -272,6 +298,8 @@ def run_frx(args, rank, world, local_rank):
     clocks.stop()
     gpu_launches = eng.launches - launches0
     total_ms = sum(s.elapsed_time(e) for s, e in ev)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {"logits": logits, "tokens": tokens})   # the last timed step's results
 
     # ---- timed region 2: host buffers through the public entry (e2e) ------------
     # (a) one synchronous call per batch (H2D -> encode -> decode -> D2H -> sync), (b) the pipelined entry: the same
@@ -363,20 +391,17 @@ def run_frx(args, rank, world, local_rank):
         "clocks": clocks.summary(),
     }
     if world == 1 and not args.no_cpu_baseline:
-        # CPU leg (the only place bench.py touches oracle/): the oracle's op-for-op port of the reference's CPU
-        # algorithm, timed on a bounded sample, on the BatchNorm-calibrated synthetic checkpoint of the parity
-        # tests (plain random-init weights are numerically degenerate, SURVEY F5), and the token agreement of
-        # both GPU modes with it on the same images.
-        from oracle import satrn as o_satrn, synth as o_synth
+        # CPU leg: the oracle's op-for-op port of the reference's CPU algorithm, timed on a bounded sample, on the
+        # checkpoint the GPU arm runs, and the token agreement of both GPU modes with it on the same images.
+        from oracle import satrn as o_satrn
         import frx
         from helpers import Vocab, flags_dict
-        sd_cal = o_synth.synth_state_dict(o_satrn.ModelSpec(), 0)
-        ips, cores, cpu_tok, dt = cpu_reference_throughput(sd_cal, args.cpu_sample, args.cpu_runs)
+        ips, cores, cpu_tok, dt = cpu_reference_throughput(sd, args.cpu_sample, args.cpu_runs)
         xs = synthetic_images(args.cpu_sample, 0).to(dev)
         agree = {}
         with torch.no_grad():
             for prec in ("fp32", "bf16"):
-                m = frx.EfficientSATRN(frx.Flags(flags_dict()).get(), Vocab(), sd_cal, None, precision=prec,
+                m = frx.EfficientSATRN(frx.Flags(flags_dict()).get(), Vocab(), sd, None, precision=prec,
                                        max_batch=args.cpu_sample, max_steps=T).to(dev).eval()
                 _, tok = m.greedy(xs, T)
                 agree[prec] = (tok.cpu() == cpu_tok).float().mean().item()
@@ -385,7 +410,7 @@ def run_frx(args, rank, world, local_rank):
         try:
             torch.backends.cuda.matmul.allow_tf32 = False
             torch.backends.cudnn.allow_tf32 = False
-            sd_gpu = {k: (v.float() if v.is_floating_point() else v).to(dev) for k, v in sd_cal.items()}
+            sd_gpu = {k: (v.float() if v.is_floating_point() else v).to(dev) for k, v in sd.items()}
             xg = synthetic_images(B, 0).to(dev)
             with torch.no_grad():
                 o_satrn.forward_greedy(sd_gpu, o_satrn.ModelSpec(), xg[:8], 8, as_written=True)
@@ -438,12 +463,12 @@ def _timed(step, steps, warmup, dev, world, flush):
     for s, e in ev:
         flush.zero_()
         s.record()
-        step()
+        last = step()
         e.record()
     if world > 1:
         dist.barrier()
     torch.cuda.synchronize(dev)
-    return sum(s.elapsed_time(e) for s, e in ev), t_begin, time.monotonic()
+    return sum(s.elapsed_time(e) for s, e in ev), t_begin, time.monotonic(), last
 
 
 def run_workload(args, rank, world, local_rank):
@@ -471,6 +496,7 @@ def run_workload(args, rank, world, local_rank):
         x, e = x_host.to(dev), e_host.to(dev)
         eng = model.engine(dev, B, T)
         step_device = lambda: model.train_step(x, e)
+        outputs = lambda last: {"loss": last[0], "grad_norm": last[1]}
 
         def step_host():
             loss, _ = model.train_step(x_host.to(dev, non_blocking=True), e_host.to(dev, non_blocking=True))
@@ -489,6 +515,7 @@ def run_workload(args, rank, world, local_rank):
         x = x_host.to(dev)
         eng = model.engine(dev, B, T)
         step_device = lambda: model.beam_search(x, None, 1, width, MAX_SEQUENCE)    # returns the tokens on the host
+        outputs = lambda last: {"tokens": last}
         step_host = lambda: model.beam_search(x_host.to(dev, non_blocking=True), None, 1, width, MAX_SEQUENCE)
         h2d, d2h = x_host.numel() * 4, B * MAX_SEQUENCE * 8
         metric = "EfficientSATRN beam-search (width %d) images/sec" % width
@@ -509,6 +536,7 @@ def run_workload(args, rank, world, local_rank):
         eng = model.engine(dev, B, T)
         tok = torch.empty(B, T, dtype=torch.int64, device=dev)
         step_device = lambda: eng.h.call("frx_forward_greedy", x.data_ptr(), B, T, None, tok.data_ptr(), torch.cuda.current_stream(dev).cuda_stream)
+        outputs = lambda last: {"tokens": tok}
         step_host = lambda: model.greedy(x_host.to(dev, non_blocking=True), T, want_logits=False)[1].cpu()
         h2d, d2h = x_host.numel() * 4, B * T * 8
         metric = "LiteSATRN greedy-decode images/sec"
@@ -525,6 +553,7 @@ def run_workload(args, rank, world, local_rank):
         eng = model.engine(dev, B, T)
         tok = torch.empty(B, T, dtype=torch.int64, device=dev)
         step_device = lambda: eng.h.call("frx_forward_greedy", x.data_ptr(), B, T, None, tok.data_ptr(), torch.cuda.current_stream(dev).cuda_stream)
+        outputs = lambda last: {"tokens": tok}
         step_host = lambda: model.greedy(x_host.to(dev, non_blocking=True), T, want_logits=False)[1].cpu()
         h2d, d2h = x_host.numel() * 4, B * T * 8
         metric = "SwinTRN greedy-decode images/sec"
@@ -533,7 +562,9 @@ def run_workload(args, rank, world, local_rank):
         dtype = "bf16" if args.precision == "bf16" else "f32"
 
     launches0 = eng.launches
-    total_ms, t0, t1 = _timed(step_device, args.steps, args.warmup, dev, world, flush)
+    total_ms, t0, t1, last = _timed(step_device, args.steps, args.warmup, dev, world, flush)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, outputs(last))
     clocks.t0, clocks.t1 = t0, t1
     clocks.stop()
     gpu_launches = eng.launches - launches0
@@ -695,7 +726,13 @@ def main():
     ap.add_argument("--cpu-sample", type=int, default=32)
     ap.add_argument("--cpu-runs", type=int, default=8)
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step computed (rank 0) as DIR/<name>.npy, under 64 MB in all")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs applies to --impl frx")
     if args.workload == "greedy" and not args.batch:
         args.batch = 256
     rank = int(os.environ.get("RANK", "0"))

@@ -20,14 +20,25 @@ oracle/make_golden.py), by the oracle and by the CUDA library.
 """
 from __future__ import annotations
 
+import hashlib
 import os
+import tempfile
 from typing import Dict
 
 import torch
 
 from . import satrn
 
-_CACHE_DIR = os.path.join(os.path.dirname(os.path.abspath(__file__)), "_cache")
+
+def _cache_dir() -> str:
+    """Per-user directory under the system temporary directory, never inside the repository (which may be
+    read-only).  Its name carries a hash of this file and of oracle/satrn.py (the BatchNorm calibration forward), so
+    a checkpoint cached by other code is never loaded."""
+    h = hashlib.sha256()
+    for f in (__file__, satrn.__file__):
+        with open(f, "rb") as fh:
+            h.update(fh.read())
+    return os.path.join(tempfile.gettempdir(), "frx-synth-%d-%s" % (os.getuid(), h.hexdigest()[:16]))
 
 
 def _draw(name: str, shape: tuple, g: torch.Generator) -> torch.Tensor:
@@ -59,8 +70,10 @@ def _draw(name: str, shape: tuple, g: torch.Generator) -> torch.Tensor:
 def synth_state_dict(spec: satrn.ModelSpec, seed: int = 0, calib_batch: int = 8,
                      cache: bool = True) -> Dict[str, torch.Tensor]:
     tag = "%s_%dx%dx%d_s%d_b%d.pt" % (spec.network, spec.in_ch, spec.height, spec.width, seed, calib_batch)
-    path = os.path.join(_CACHE_DIR, tag)
-    if cache and os.path.exists(path):
+    cache_dir = _cache_dir()
+    path = os.path.join(cache_dir, tag)
+    # only a directory this user owns is trusted (the temporary directory is shared)
+    if cache and os.path.exists(path) and os.stat(cache_dir).st_uid == os.getuid():
         return torch.load(path)
     g = torch.Generator().manual_seed(1000 + seed)
     sd = {n: _draw(n, s, g) for n, s in satrn.param_shapes(spec).items()}
@@ -70,10 +83,13 @@ def synth_state_dict(spec: satrn.ModelSpec, seed: int = 0, calib_batch: int = 8,
     with torch.no_grad():
         satrn.encoder_forward(sd, spec, imgs, calib=satrn._Calib(sd))
     if cache:
-        os.makedirs(_CACHE_DIR, exist_ok=True)
-        tmp = path + ".%d.tmp" % os.getpid()
-        torch.save(sd, tmp)
-        os.replace(tmp, path)
+        try:
+            os.makedirs(cache_dir, mode=0o700, exist_ok=True)
+            tmp = path + ".%d.tmp" % os.getpid()
+            torch.save(sd, tmp)
+            os.replace(tmp, path)
+        except OSError:
+            pass    # the cache only saves time
     return sd
 
 
