@@ -97,6 +97,25 @@ int frx_decode_greedy(frx_handle* h, const float* memory, int32_t batch, int32_t
 int frx_forward_greedy(frx_handle* h, const float* images, int32_t batch, int32_t steps,
                        float* logits, int64_t* tokens, void* stream);
 
+/* Greedy decode that stops each image at its first <EOS> (what id_to_string keeps, utils/utils.py:134-164), opt-in.
+ * len[b] = index of the first emitted <EOS> + 1 (emitted: the arg-max, or with managed != 0 the DecodingManager's pick
+ * -- the token frx_decode_greedy writes to `tokens`), or max_steps if there is none.  With `forced`, row b stops after
+ * the step t at which forced[b, t] == <EOS> instead.
+ * logits  : device fp32 [B, max_steps, num_classes] (managed: masked softmax rows) or NULL.  Rows t < len[b] are
+ *           bit-identical to frx_decode_greedy's (frx_decode_greedy_managed's) on the same handle and batch; rows
+ *           t >= len[b] are 0.
+ * tokens  : device int64 [B, max_steps] or NULL: the full decode's tokens for t < len[b], <PAD> after.
+ * lengths : device int32 [B].
+ * Errors as frx_decode_greedy / frx_decode_greedy_managed (managed with forced is rejected).  The 16-bit persistent
+ * decode kernel stops the work of an image at its <EOS> and hands its cluster row the next image; fp32 mode and 16-bit
+ * handles on the step kernels decode all max_steps and apply the same contract afterwards (same output, no time saved).
+ * Enqueues work only (no synchronisation), so it can be captured in a CUDA graph. */
+int frx_decode_greedy_eos(frx_handle* h, const float* memory, int32_t batch, int32_t max_steps, float* logits,
+                          int64_t* tokens, int32_t* lengths, const int64_t* forced, int32_t managed, void* stream);
+/* frx_encode + frx_decode_greedy_eos. */
+int frx_forward_greedy_eos(frx_handle* h, const float* images, int32_t batch, int32_t max_steps, float* logits,
+                           int64_t* tokens, int32_t* lengths, int32_t managed, void* stream);
+
 /* Same call with HOST buffers (pinned or pageable): H2D of the images, encode,
  * decode, D2H of tokens (and of logits when logits_host != NULL); synchronises
  * the stream before returning.  This is the end-to-end entry bench.py times. */

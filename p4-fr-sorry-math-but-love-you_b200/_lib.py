@@ -17,6 +17,7 @@ SYMBOLS = [
     "frx_train_create", "frx_train_destroy", "frx_train_param_count", "frx_train_fwd_bwd", "frx_train_grad_buffer",
     "frx_train_set_bucket_callback", "frx_train_apply", "frx_train_export", "frx_train_read_grad", "frx_train_step_count", "frx_train_read_tap",
     "frx_train_forward", "frx_train_backward", "frx_train_import", "frx_ensemble_decode", "frx_preprocess_u8", "frx_train_apply_dual",
+    "frx_decode_greedy_eos", "frx_forward_greedy_eos",
 ]
 
 BUCKET_CALLBACK = ctypes.CFUNCTYPE(None, ctypes.c_void_p, ctypes.c_int64, ctypes.c_int64)
@@ -78,6 +79,8 @@ def load_library():
     lib.frx_set_decoding_rules.argtypes = [vp, ctypes.POINTER(i32), ctypes.POINTER(i32), i32, ctypes.POINTER(i32)]
     lib.frx_decode_greedy_managed.argtypes = [vp, vp, i32, i32, vp, vp, vp]
     lib.frx_forward_greedy_managed.argtypes = [vp, vp, i32, i32, vp, vp, vp]
+    lib.frx_decode_greedy_eos.argtypes = [vp, vp, i32, i32, vp, vp, vp, vp, i32, vp]
+    lib.frx_forward_greedy_eos.argtypes = [vp, vp, i32, i32, vp, vp, vp, i32, vp]
     f32 = ctypes.c_float
     lib.frx_train_create.argtypes = [vp, i32, i32, vp]
     lib.frx_train_destroy.argtypes = [vp]

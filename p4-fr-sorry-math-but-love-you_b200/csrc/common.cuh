@@ -253,6 +253,12 @@ struct DecClusterP {
   const int* sift_limit;
   SiftIds sift_ids;
   long long* prof;               // optional [16] per-stage cycle totals (cluster 0, CTA 0, thread 0)
+  // stop-at-<EOS> instantiations (FRX_DEC_EOS): each of a cluster's rows decodes one image until it emits `eos` (forced:
+  // until forced[b][t] == eos) or reaches `steps`, writes lengths[b] = steps decoded, and takes the next image from the
+  // zeroed counter *work.  The self K/V caches are indexed by slot (cluster * 8 + row) instead of by image.
+  int* lengths;                  // [B] int32
+  int* work;                     // images handed out so far (zero before the launch)
+  int eos;
 };
 
 }  // namespace frx

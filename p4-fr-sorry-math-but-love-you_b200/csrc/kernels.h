@@ -38,6 +38,8 @@ void launch_dec_sift_embed(float* logits, long long ld_logits, int V, long long*
                            const float* pe_next, float scale, float* x, int M, int D, cudaStream_t st);
 void launch_sift_state_init(int4* state, int M, int sos, cudaStream_t st);
 void launch_pad_mask(const long long* text, unsigned char* mask, int B, int L, int pad_id, cudaStream_t st);
+void launch_eos_finalize(float* logits, long long* tokens, int* lengths, const long long* stop, int B, int steps, int V,
+                         int eos, int pad, bool have_len, cudaStream_t st);
 
 // SwinTRN encoder pieces (kernels_swin.cu)
 void launch_swin_patch_embed(const float* img, const float* w, const float* bias, const float* g, const float* b,
@@ -87,6 +89,11 @@ int launch_dec_cluster_bf16(const DecClusterP& p, cudaStream_t st);       // hid
 int launch_dec_cluster_bf16_d128(const DecClusterP& p, cudaStream_t st);  // hidden 128, 4 heads, filter 512 (clusters of 4)
 int launch_dec_cluster_bf16_p2(const DecClusterP& p, cudaStream_t st);    // hidden 256, two heads per CTA (clusters of 4 x 16 warps)
 int launch_dec_cluster_bf16_d512(const DecClusterP& p, cudaStream_t st);  // hidden 512, 8 heads x 64, filter 512 (SwinTRN decoder)
+// stop-at-<EOS> instantiations of the four geometries (DecClusterP::lengths / work / eos): one launch for any batch
+int launch_dec_cluster_bf16_eos(const DecClusterP& p, cudaStream_t st);
+int launch_dec_cluster_bf16_d128_eos(const DecClusterP& p, cudaStream_t st);
+int launch_dec_cluster_bf16_p2_eos(const DecClusterP& p, cudaStream_t st);
+int launch_dec_cluster_bf16_d512_eos(const DecClusterP& p, cudaStream_t st);
 void launch_cross_to_bf16(const float* src, __nv_bfloat16* kc, __nv_bfloat16* vc, int B, int S, int L, int Dm, int head_dim,
                           cudaStream_t st);
 

@@ -73,6 +73,11 @@ constexpr bool KV_BULK = FRX_DEC_KVBULK;
 #define FRX_DEC_EARLYPRIME FRX_DEC_KVBULK   // request the next attention phase's first K/V blocks as soon as the ring is idle (measured: pays with the bulk-copy ring only)
 #endif
 constexpr bool EARLY_PRIME = FRX_DEC_EARLYPRIME;
+#ifdef FRX_DEC_EOS
+constexpr bool EOS = true;       // rows stop at <EOS> and are refilled with the next image (kernels_decode_bf16*_eos.cu)
+#else
+constexpr bool EOS = false;
+#endif
 constexpr int CL = H / HPC;      // CTAs per cluster
 constexpr int FF = FRX_DEC_FF;
 constexpr int VP = 256;          // vocabulary columns, padded
@@ -142,6 +147,17 @@ struct Smem {
   unsigned long long kvbar[NWARP][KVD]; // per-warp mbarriers of the K/V ring slots (bulk copies of contiguous histories)
   DecClusterLayer lw[4];                // per-layer pointers (dynamic indexing of kernel params would spill them)
 };
+// Per-row state of the stop-at-<EOS> instantiations, in shared memory behind Smem (the two-heads geometry has no
+// registers to spare for it).
+struct EosRows {
+  int img[NIMG];                        // image each row decodes (-1: idle, no work left)
+  int pos[NIMG];                        // its position = the step it is at
+  int done[NIMG];                       // the row finished its image at this step
+  int left[NIMG];                       // history length of the image a refilled row left (its early-primed K/V blocks)
+  int claim[8];                         // claim[c]: what CTA c sent in this step's refill exchange (rank 0: first image)
+};
+constexpr size_t SMEM_BYTES = sizeof(Smem) + (EOS ? sizeof(EosRows) : 0);
+static_assert(!(EOS && EARLY_PRIME) || KV_BULK, "a refilled row drains the early-primed blocks on the ring's mbarriers");
 
 // ---------------------------------------------------------------------------
 // GEMM stage: out[8 images, NT*8 columns of this CTA] = A[8, K] * W^T; A bf16 in smem (rows 8..15 of the
@@ -657,6 +673,7 @@ __global__ void __cluster_dims__(CL, 1, 1) __launch_bounds__(NTHR, FRX_DEC_MINBL
 FRX_DEC_NAME(dec_cluster_bf16_kernel)(const DecClusterP p) {
   extern __shared__ __align__(16) unsigned char smem_raw[];
   Smem& s = *reinterpret_cast<Smem*>(smem_raw);
+  EosRows& er = *reinterpret_cast<EosRows*>(smem_raw + sizeof(Smem));   // stop-at-<EOS> instantiations only
   cg::cluster_group cl = cg::this_cluster();
   const int r = (int)cl.block_rank();                        // CTA rank = head index = column slice
   const int img0 = p.img_base + (blockIdx.x / CL) * NIMG;    // first image of this cluster
@@ -735,13 +752,48 @@ FRX_DEC_NAME(dec_cluster_bf16_kernel)(const DecClusterP p) {
   };
   const int wimg = warp % NIMG, whc = warp / NIMG;  // this warp attends for image wimg, head r * HPC + whc
   const int head = r * HPC + whc;
-  const int b_mine = img0 + wimg;
-  const bool mine = b_mine < B;
+  int b_mine = img0 + wimg;     // stop-at-<EOS>: the row's current image (-1: idle), re-read every step
+  bool mine = b_mine < B;
   const int hist0 = (mine && p.hist_len) ? __ldg(p.hist_len + b_mine) : 0;      // keys cached before this launch
   const int* const chain = (mine && p.chain) ? p.chain + (size_t)b_mine * T : nullptr;
   KVStage* const kvst = reinterpret_cast<KVStage*>(&s.kvst[warp][0][0][0][0]);  // this warp's ring of K/V staging blocks
   const uint32_t kvbar = smem_u32(&s.kvbar[warp][0]);
   uint32_t kvphase = 0;   // bit d: parity of the next completion of ring slot d
+  // Self K/V caches: [L][B][H][T][HD] by image, or (stop-at-<EOS>) [L][NSL][H][T][HD] by slot = cluster * 8 + row over all
+  // of the launch's slots: any cluster may claim any image, so every slot may decode.  The grid has at most ceil(B / 8)
+  // clusters, and the 16-bit self caches are allocated for max_batch rounded up to a multiple of 8.
+  const int NSL = EOS ? (int)(gridDim.x / CL) * NIMG : B;
+  const int kslot = EOS ? img0 + wimg : b_mine;   // cache slot of this warp's row
+
+  // Stop-at-<EOS>: rows whose bit is set in `mask` take the next images from the work counter.  Every CTA of the cluster
+  // takes the same decisions (the picks run on the gathered logits), so only the claimed index travels: rank 0 claims
+  // one image per row and sends the first index on the stage mbarrier -- an exchange on steps where a row finished only.
+  // Every CTA sends its word to every CTA (the others a dummy), so that, as for every other exchange, a CTA's wait ends
+  // only when all its peers have reached the exchange: with rank 0 alone sending, a CTA could run two exchanges ahead of
+  // a peer still waiting for the logits and complete that peer's barrier phase with the next step's stores.
+  // Refilled rows restart at <SOS>, position 0, with a fresh MemoryNode state.
+  auto refill = [&](uint32_t mask) {
+    stage_begin(4u * CL);
+    if (tid == 0) {
+      const int first = r == 0 ? atomicAdd(p.work, __popc(mask)) : 0;
+      for (int d = 0; d < CL; ++d) st_async_b32(mapa_u32(smem_u32(&er.claim[r]), d), (uint32_t)first, mapa_u32(stage_bar(), d));
+    }
+    stage_end();
+    if (tid < NIMG && ((mask >> tid) & 1u)) {
+      const int img = er.claim[0] + __popc(mask & ((1u << tid) - 1u));
+      er.img[tid] = img < B ? img : -1;
+      er.left[tid] = er.pos[tid] + 1;
+      er.pos[tid] = 0;
+      s.sift[tid] = make_int4(p.sift_ids.sos, 1, 0, 0);
+    }
+    for (int i = tid; i < NIMG * D; i += NTHR) {
+      const int row = i / D, c = i % D;
+      if (!((mask >> row) & 1u)) continue;
+      const float v = __ldg(p.emb + (size_t)p.sos * D + c) * emb_scale + __ldg(p.pe + c);
+      s.xres[row][c] = v;
+      s.abf[row][c] = __float2bfloat16_rn(v);
+    }
+  };
 
   // all-gather of this warp's attention output (head r, image `warp`) into every CTA's obf: the eight gid
   // groups of the warp hold identical copies, group g serves destination CTA g
@@ -809,13 +861,14 @@ FRX_DEC_NAME(dec_cluster_bf16_kernel)(const DecClusterP p) {
   auto cache_rows = [&](int lc, int t, const uint4* wp, const float* bias) {
     const Bias8 cb = ldg_bias8(bias + ((tid >> 3) / NTS) * D + r * SW + ((tid >> 3) % NTS) * 8, tid < NTC * 8);
     gemm2<NTC, KPD, KS>(next_red(), &s.abf[0][0], LDA, wp, pol, WPre<0>{}, [&](int tile, int row, float (&v)[8], int sub) {
-      const int b = img0 + row;
-      if (sub != 0 || b >= B) return;
+      const int b = img0 + row;   // stop-at-<EOS>: the row's slot
+      if (sub != 0 || (EOS ? er.img[row] < 0 : b >= B)) return;
       const int seg = tile / NTS, wc = (tile % NTS) * 8, hd = r * HPC + wc / HD, col = wc % HD;
       const float4 b0 = cb.a, b1 = cb.b;
       __nv_bfloat16* dst = seg == 0 ? p.kself : p.vself;
-      const int wrow = (p.slot ? __ldg(p.slot + b) : (p.hist_len ? __ldg(p.hist_len + b) : 0)) + t;   // cache row of this step
-      *reinterpret_cast<uint4*>(dst + (((((size_t)lc * B + b) * H + hd) * T) + wrow) * HD + (((col >> 3) ^ kv_perm(wrow)) << 3)) =
+      const int wrow = EOS ? er.pos[row]
+                           : (p.slot ? __ldg(p.slot + b) : (p.hist_len ? __ldg(p.hist_len + b) : 0)) + t;   // cache row of this step
+      *reinterpret_cast<uint4*>(dst + (((((size_t)lc * NSL + b) * H + hd) * T) + wrow) * HD + (((col >> 3) ^ kv_perm(wrow)) << 3)) =
           make_uint4(pack_bf16(v[0] + b0.x, v[1] + b0.y), pack_bf16(v[2] + b0.z, v[3] + b0.w),
                      pack_bf16(v[4] + b1.x, v[5] + b1.y), pack_bf16(v[6] + b1.z, v[7] + b1.w));
       // the row is read back by bulk copies (async proxy) from the next step on: order this generic-proxy write before them
@@ -829,23 +882,52 @@ FRX_DEC_NAME(dec_cluster_bf16_kernel)(const DecClusterP p) {
   // the next layer (next step: layer 0, whose newest cache row was written during this step's layer 1) right after the
   // cross-attention -- they land under the stages in between instead of under one short projection.
   auto prime_self = [&](int l, int t) {
-    const size_t base = ((((size_t)l * B + (mine ? b_mine : 0)) * H + head) * T) * HD;
+    const size_t base = ((((size_t)l * NSL + (mine ? kslot : 0)) * H + head) * T) * HD;
     kv_prime(kvst, p.kself + base, p.vself + base, mine ? hist0 + t : 0, chain, kvbar);
   };
   auto prime_cross = [&](int l) {
     const size_t base = ((((size_t)l * B + (mine ? b_mine : 0)) * H + head) * p.S) * HD;
     kv_prime(kvst, p.kcross + base, p.vcross + base, mine ? p.S : 0, nullptr, kvbar);
   };
+  if constexpr (EOS) {   // every row starts with a claimed image
+    if (tid < NIMG) { er.pos[tid] = 0; er.done[tid] = 0; }
+    refill(0xffu);
+    __syncthreads();
+    b_mine = er.img[wimg];
+    mine = b_mine >= 0;
+  }
   prime_self(0, 0);
   bool self_primed = true;
-  for (int t = 0; t < p.steps; ++t) {
+  for (int t = 0; EOS || t < p.steps; ++t) {
+    // position of this warp's row, re-read where it is used (a register for it through the step would spill)
+    const auto tpos = [&]() { return EOS ? er.pos[wimg] : t; };
+    if constexpr (EOS) {
+      b_mine = er.img[wimg];
+      mine = b_mine >= 0;
+    }
     for (int l = 0; l < L; ++l) {
       const DecClusterLayer& W = s.lw[l];
       // ---- A: q|k|v of head r from the layer input, then self attention of (image warp, head r) -------
       {
-        const size_t base = ((((size_t)l * B + (mine ? b_mine : 0)) * H + head) * T) * HD;
-        const int n_hist = mine ? hist0 + t : 0;
-        if (!self_primed) prime_self(l, t);   // single-layer decoders only: the newest cache row is written late in the step
+        const size_t base = ((((size_t)l * NSL + (mine ? kslot : 0)) * H + head) * T) * HD;
+        const int n_hist = mine ? hist0 + tpos() : 0;
+        if constexpr (EOS && EARLY_PRIME) {
+          // the blocks requested for this step at the end of the last one belong to a history the row has left (it
+          // finished, was refilled or went idle): let them land, then request the row's own
+          if (l == 0 && self_primed && er.done[wimg]) {
+            const int primed_n = er.left[wimg];   // what the last step's early prime requested (mine: the row was busy)
+#pragma unroll
+            for (int d = 0; d < KVD; ++d) {
+              if (32 * d < primed_n) {
+                mbar_wait(kvbar + 8u * d, (kvphase >> d) & 1u);
+                kvphase ^= 1u << d;
+              }
+            }
+            __syncwarp();
+            self_primed = false;
+          }
+        }
+        if (!self_primed) prime_self(l, tpos());   // single-layer decoders only: the newest cache row is written late in the step
         self_primed = false;
         const uint4* wp = l == 0 ? p.w_first + (size_t)r * NTA * WT : s.lw[l - 1].w_next + ((size_t)r * (NTC + NTA) + NTC) * WT;
         const Bias8 bias = qkv_bias(l == 0 ? p.b_first : s.lw[l - 1].b_next + 2 * D);
@@ -910,8 +992,11 @@ FRX_DEC_NAME(dec_cluster_bf16_kernel)(const DecClusterP p) {
         }
         store_attn(sb, o);
         if (EARLY_PRIME) {
-          if (l + 1 < L) { prime_self(l + 1, t); self_primed = true; }
-          else if (L >= 2 && t + 1 < p.steps) { prime_self(0, t + 1); self_primed = true; }
+          if (l + 1 < L) { prime_self(l + 1, tpos()); self_primed = true; }
+          else if (L >= 2 && (EOS || t + 1 < p.steps)) {
+            prime_self(0, tpos() + 1);
+            self_primed = true;
+          }
         }
         mark(7);
       }
@@ -1004,9 +1089,9 @@ FRX_DEC_NAME(dec_cluster_bf16_kernel)(const DecClusterP p) {
                               st_async_v4(la, make_uint4(__float_as_uint(v[0]), __float_as_uint(v[1]), __float_as_uint(v[2]), __float_as_uint(v[3])), rb);
                               st_async_v4(la + 16, make_uint4(__float_as_uint(v[4]), __float_as_uint(v[5]), __float_as_uint(v[6]), __float_as_uint(v[7])), rb);
                             }
-                            const int b = img0 + row;
-                            if (sub == (CL > 1 ? 1 : 0) && p.logits && b < B && !p.sift_flags) {
-                              float* lp = p.logits + ((size_t)b * p.steps + t) * V + col;
+                            const int b = EOS ? er.img[row] : img0 + row;
+                            if (sub == (CL > 1 ? 1 : 0) && p.logits && (EOS ? b >= 0 : b < B) && !p.sift_flags) {
+                              float* lp = p.logits + ((size_t)b * p.steps + (EOS ? er.pos[row] : t)) * V + col;
 #pragma unroll
                               for (int i = 0; i < 8; ++i)
                                 if (col + i < V) lp[i] = v[i];
@@ -1025,7 +1110,7 @@ FRX_DEC_NAME(dec_cluster_bf16_kernel)(const DecClusterP p) {
       const int row = warp;
       int bi;
       if (p.sift_flags) {
-        float* prow = (mine && r == 0 && p.logits) ? p.logits + ((size_t)b_mine * p.steps + t) * V : nullptr;
+        float* prow = (mine && r == 0 && p.logits) ? p.logits + ((size_t)b_mine * p.steps + tpos()) * V : nullptr;
         bi = sift_pick(logit_s + row * LGS, V, &s.sift[row], p.sift_flags, p.sift_limit, p.sift_ids, prow);
       } else {
         float best = -INFINITY;
@@ -1044,11 +1129,17 @@ FRX_DEC_NAME(dec_cluster_bf16_kernel)(const DecClusterP p) {
       }
       int nxt = bi;
       if (mine) {
-        if (p.forced) nxt = (int)p.forced[(size_t)b_mine * p.steps + t];
-        if (r == 0 && lane == 0 && p.tokens) p.tokens[(size_t)b_mine * p.steps + t] = bi;
+        if (p.forced) nxt = (int)p.forced[(size_t)b_mine * p.steps + tpos()];
+        if (r == 0 && lane == 0 && p.tokens) p.tokens[(size_t)b_mine * p.steps + tpos()] = bi;
       }
-      if (t + 1 < p.steps) {
-        const float* pe = p.pe + (size_t)(hist0 + t + 1) * D;
+      bool more = t + 1 < p.steps;
+      if constexpr (EOS) {   // the row stops after the step that emits (forced: is fed) <EOS>, or after the last step
+        more = mine && nxt != p.eos && tpos() + 1 < p.steps;
+        if (mine && !more && r == 0 && lane == 0) p.lengths[b_mine] = tpos() + 1;
+        if (lane == 0) er.done[row] = mine && !more;
+      }
+      if (more) {
+        const float* pe = p.pe + (size_t)(hist0 + tpos() + 1) * D;
 #pragma unroll
         for (int i = 0; i < D / 32; ++i) {
           const int c = i * 32 + lane;
@@ -1060,24 +1151,42 @@ FRX_DEC_NAME(dec_cluster_bf16_kernel)(const DecClusterP p) {
     }
     __syncthreads();
     mark(10);
+    if constexpr (EOS) {
+      uint32_t finished = 0;
+#pragma unroll
+      for (int i = 0; i < NIMG; ++i) finished |= (er.done[i] ? 1u : 0u) << i;
+      if (tid < NIMG && er.img[tid] >= 0 && !((finished >> tid) & 1u)) er.pos[tid] += 1;
+      if (finished) refill(finished);
+      __syncthreads();
+      bool busy = false;
+#pragma unroll
+      for (int i = 0; i < NIMG; ++i) busy = busy || er.img[i] >= 0;
+      if (!busy) break;   // the same decision in every CTA of the cluster
+    }
   }
   cl.sync();  // nobody exits while a peer's stores to it may still be in flight
   if (profiling) for (int i = 0; i < 16; ++i) p.prof[i] = s.prof[i];
 }
 
-size_t FRX_DEC_NAME(dec_cluster_smem_bytes)() { return sizeof(Smem); }
+size_t FRX_DEC_NAME(dec_cluster_smem_bytes)() { return SMEM_BYTES; }
 
 // One launch decodes up to DEC_MAX_CLUSTERS clusters (all co-resident: two CTAs per SM); larger batches
-// are decoded in consecutive launches over image ranges.
+// are decoded in consecutive launches over image ranges.  The stop-at-<EOS> instantiations decode any batch in one
+// launch of at most DEC_MAX_CLUSTERS clusters whose rows take images from the work counter.
 int FRX_DEC_NAME(launch_dec_cluster_bf16)(const DecClusterP& p0, cudaStream_t st) {
   static SmemOptIn opt;
   {
-    cudaError_t e = opt.ensure(FRX_DEC_NAME(dec_cluster_bf16_kernel), sizeof(Smem), true);
+    cudaError_t e = opt.ensure(FRX_DEC_NAME(dec_cluster_bf16_kernel), SMEM_BYTES, true);
     if (e != cudaSuccess) return (int)e;
+  }
+  if (EOS) {
+    const int clusters = (p0.B + NIMG - 1) / NIMG < DEC_MAX_CLUSTERS ? (p0.B + NIMG - 1) / NIMG : DEC_MAX_CLUSTERS;
+    FRX_DEC_NAME(dec_cluster_bf16_kernel)<<<clusters * CL, NTHR, SMEM_BYTES, st>>>(p0);
+    return 0;
   }
   if (getenv("FRX_DEBUG")) {
     cudaLaunchConfig_t cfg{};
-    cfg.gridDim = dim3(DEC_MAX_CLUSTERS * CL); cfg.blockDim = dim3(NTHR); cfg.dynamicSmemBytes = sizeof(Smem);
+    cfg.gridDim = dim3(DEC_MAX_CLUSTERS * CL); cfg.blockDim = dim3(NTHR); cfg.dynamicSmemBytes = SMEM_BYTES;
     cudaLaunchAttribute at[1];
     at[0].id = cudaLaunchAttributeClusterDimension;
     at[0].val.clusterDim.x = CL; at[0].val.clusterDim.y = 1; at[0].val.clusterDim.z = 1;
@@ -1085,14 +1194,14 @@ int FRX_DEC_NAME(launch_dec_cluster_bf16)(const DecClusterP& p0, cudaStream_t st
     int n = -1;
     cudaError_t e = cudaOccupancyMaxActiveClusters(&n, FRX_DEC_NAME(dec_cluster_bf16_kernel), &cfg);
     fprintf(stderr, "[frx] decode kernel: clusters of %d CTAs x %d threads, max co-resident clusters = %d (%s), smem %zu B\n",
-            CL, NTHR, n, cudaGetErrorString(e), sizeof(Smem));
+            CL, NTHR, n, cudaGetErrorString(e), SMEM_BYTES);
   }
   for (int base = 0; base < p0.B; base += DEC_MAX_CLUSTERS * NIMG) {
     DecClusterP p = p0;
     p.img_base = base;
     const int n = p0.B - base < DEC_MAX_CLUSTERS * NIMG ? p0.B - base : DEC_MAX_CLUSTERS * NIMG;
     const int clusters = (n + NIMG - 1) / NIMG;
-    FRX_DEC_NAME(dec_cluster_bf16_kernel)<<<clusters * CL, NTHR, sizeof(Smem), st>>>(p);
+    FRX_DEC_NAME(dec_cluster_bf16_kernel)<<<clusters * CL, NTHR, SMEM_BYTES, st>>>(p);
   }
   return 0;
 }

@@ -1002,6 +1002,34 @@ void launch_pad_mask(const long long* text, unsigned char* mask, int B, int L, i
   pad_mask_kernel<<<(B * L + 255) / 256, 256, 0, st>>>(text, mask, B, L, pad_id);
 }
 
+// Stop-at-<EOS> contract on a greedy result (one block per image): len = index of the first `eos` in stop[b] + 1, or
+// steps; tokens after it become `pad`, logits rows after it 0.  have_len: lengths[b] is given (the stop-at-<EOS> kernel
+// wrote only the rows up to it), else it is found in stop[] (the tokens, or the forced sequence) and written.
+__global__ void __launch_bounds__(256) eos_finalize_kernel(float* __restrict__ logits, long long* __restrict__ tokens,
+                                                           int* __restrict__ lengths, const long long* __restrict__ stop,
+                                                           int steps, int V, int eos, int pad, int have_len) {
+  __shared__ int first;
+  const int b = blockIdx.x;
+  if (threadIdx.x == 0) first = steps;
+  __syncthreads();
+  if (!have_len) {
+    for (int t = threadIdx.x; t < steps; t += blockDim.x)
+      if (stop[(size_t)b * steps + t] == eos) atomicMin(&first, t + 1);
+    __syncthreads();
+    if (threadIdx.x == 0) lengths[b] = first;
+  }
+  const int len = have_len ? lengths[b] : first;
+  for (int t = len + threadIdx.x; t < steps; t += blockDim.x) tokens[(size_t)b * steps + t] = pad;
+  if (logits) {
+    float* row = logits + (size_t)b * steps * V;
+    for (size_t i = (size_t)len * V + threadIdx.x; i < (size_t)steps * V; i += blockDim.x) row[i] = 0.f;
+  }
+}
+void launch_eos_finalize(float* logits, long long* tokens, int* lengths, const long long* stop, int B, int steps, int V,
+                         int eos, int pad, bool have_len, cudaStream_t st) {
+  eos_finalize_kernel<<<B, 256, 0, st>>>(logits, tokens, lengths, stop, steps, V, eos, pad, have_len ? 1 : 0);
+}
+
 // ===========================================================================
 // DecodingManager.sift + MemoryNode.record/_look_back (postprocessing/postprocessing.py:193-233,
 // :303-391) fused with the next step's embedding: one warp per row.  In place: the row of logits becomes the

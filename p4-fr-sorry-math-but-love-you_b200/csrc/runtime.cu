@@ -889,9 +889,13 @@ extern "C" int frx_finalize_weights(frx_handle* h) {
     if (dev_alloc(h, &p, B * T * 8)) return 1; h->tokens_int = (long long*)p;
     if (dev_alloc(h, &p, B * T * 8)) return 1; h->forced_int = (long long*)p;
     if (dev_alloc(h, &p, B * 4)) return 1; h->cur_tok = (int*)p;
+    if (dev_alloc(h, &p, 16)) return 1; h->eos_work = (int*)p;
     if (c.precision == FRX_PREC_BF16) {
-      if (dev_alloc(h, &p, L * B * T * D * 2)) return 1; h->kself_bf = p;
-      if (dev_alloc(h, &p, L * B * T * D * 2)) return 1; h->vself_bf = p;
+      // self caches: [L][B][H][T][hd] by image, or [L][slots][H][T][hd] by cluster row in the stop-at-<EOS> decode,
+      // whose slots = clusters * 8 round the batch up to a multiple of 8
+      const size_t B8 = (B + DEC_IMG - 1) / DEC_IMG * DEC_IMG;
+      if (dev_alloc(h, &p, L * B8 * T * D * 2)) return 1; h->kself_bf = p;
+      if (dev_alloc(h, &p, L * B8 * T * D * 2)) return 1; h->vself_bf = p;
       if (dev_alloc(h, &p, L * B * S * D * 2)) return 1; h->kcross_bf = p;
       if (dev_alloc(h, &p, L * B * S * D * 2)) return 1; h->vcross_bf = p;
       if (dev_alloc(h, &p, B * S * (size_t)c.dec_src * 2)) return 1; h->mem_bf = p;
@@ -1517,8 +1521,11 @@ static int cross_kv_to_bf16(frx_handle* h, int B, cudaStream_t st) {
   return 0;
 }
 
+// eos_lengths != nullptr: the stop-at-<EOS> instantiation (one launch for the whole batch, rows refilled from a work
+// counter); it writes logits / tokens up to each image's length only.
 static int decode_greedy_bf16(frx_handle* h, int B, int steps, float* logits, long long* tokens,
-                              const long long* forced, cudaStream_t st, const ClusterStep* sm = nullptr, bool managed = false) {
+                              const long long* forced, cudaStream_t st, const ClusterStep* sm = nullptr, bool managed = false,
+                              int* eos_lengths = nullptr) {
   const frx_config& c = h->cfg;
   const float* A = h->arena;
   const int S = h->feat_h * h->feat_w, L = c.dec_layers, D = c.dec_hidden;
@@ -1559,8 +1566,16 @@ static int decode_greedy_bf16(frx_handle* h, int B, int steps, float* logits, lo
   p.logits = logits; p.tokens = tokens; p.forced = forced;
   p.prof = h->opt_prof ? h->prof : nullptr;
   if (p.prof) CK(cudaMemsetAsync(h->prof, 0, 16 * 8, st));
+  if (eos_lengths) {
+    p.lengths = eos_lengths; p.work = h->eos_work; p.eos = c.eos_id;
+    CK(cudaMemsetAsync(h->eos_work, 0, sizeof(int), st));
+  }
   if (h->opt_timing) CK(cudaEventRecord(h->ev[3], st));
-  int rc = D == 128 ? launch_dec_cluster_bf16_d128(p, st)
+  int rc = eos_lengths
+               ? (D == 128 ? launch_dec_cluster_bf16_d128_eos(p, st)
+                           : D == 512 ? launch_dec_cluster_bf16_d512_eos(p, st)
+                                      : (p2 ? launch_dec_cluster_bf16_p2_eos(p, st) : launch_dec_cluster_bf16_eos(p, st)))
+               : D == 128 ? launch_dec_cluster_bf16_d128(p, st)
                     : D == 512 ? launch_dec_cluster_bf16_d512(p, st) : (p2 ? launch_dec_cluster_bf16_p2(p, st) : launch_dec_cluster_bf16(p, st));
   if (rc) return fail(h, "decode cluster kernel configuration failed: %s", cudaGetErrorString((cudaError_t)rc));
   CKL();
@@ -1569,8 +1584,11 @@ static int decode_greedy_bf16(frx_handle* h, int B, int steps, float* logits, lo
   return 0;
 }
 
+// eos_lengths != nullptr: stop-at-<EOS> decode (frx_decode_greedy_eos).  The 16-bit cluster kernel stops each image at
+// its <EOS>; the other paths decode all `steps` and apply the same contract afterwards (no time saved there).
 static int decode_greedy_impl(frx_handle* h, const float* memory, int B, int steps, float* logits,
-                              int64_t* tokens, const int64_t* forced, cudaStream_t st, bool managed = false) {
+                              int64_t* tokens, const int64_t* forced, cudaStream_t st, bool managed = false,
+                              int* eos_lengths = nullptr) {
   const frx_config& c = h->cfg;
   if (!h->finalized) return fail(h, "decode: weights not finalized");
   if (!(h->opt_parts & 2)) return fail(h, "decode: handle was created without the decoder part");
@@ -1584,9 +1602,12 @@ static int decode_greedy_impl(frx_handle* h, const float* memory, int B, int ste
   const int mode = managed ? 2 : (forced ? 1 : 0);
   // bf16 mode: one persistent kernel that writes the caller's buffers directly.  Sequences longer than the kernel's
   // history capacity (the reference decodes up to the 500 rows of its 1-D positional table) take the step-kernel loop.
-  if (c.precision == FRX_PREC_BF16 && h->dec_cluster_ok && steps <= DEC_TMAX && (!managed || h->opt_step16))
-    return decode_greedy_bf16(h, B, steps, logits, (long long*)(tokens ? tokens : (int64_t*)h->tokens_int),
-                              (const long long*)forced, st, nullptr, managed);
+  if (c.precision == FRX_PREC_BF16 && h->dec_cluster_ok && steps <= DEC_TMAX && (!managed || h->opt_step16)) {
+    long long* tok = (long long*)(tokens ? tokens : (int64_t*)h->tokens_int);
+    if (decode_greedy_bf16(h, B, steps, logits, tok, (const long long*)forced, st, nullptr, managed, eos_lengths)) return 1;
+    if (eos_lengths) { launch_eos_finalize(logits, tok, eos_lengths, nullptr, B, steps, c.num_classes, c.eos_id, c.pad_id, true, st); CKL(); }
+    return 0;
+  }
   if (forced) CK(cudaMemcpyAsync(h->forced_int, forced, (size_t)B * steps * 8, cudaMemcpyDeviceToDevice, st));
   if (h->opt_graphs) {
     GraphKey key{B, steps, mode};
@@ -1627,6 +1648,12 @@ static int decode_greedy_impl(frx_handle* h, const float* memory, int B, int ste
   }
   if (logits) CK(cudaMemcpyAsync(logits, h->logits_int, (size_t)B * steps * c.num_classes * 4, cudaMemcpyDeviceToDevice, st));
   if (tokens) CK(cudaMemcpyAsync(tokens, h->tokens_int, (size_t)B * steps * 8, cudaMemcpyDeviceToDevice, st));
+  if (eos_lengths) {
+    long long* tok = (long long*)(tokens ? tokens : (int64_t*)h->tokens_int);
+    launch_eos_finalize(logits, tok, eos_lengths, forced ? (const long long*)forced : tok, B, steps, c.num_classes, c.eos_id,
+                        c.pad_id, false, st);
+    CKL();
+  }
   return 0;
 }
 
@@ -1634,6 +1661,20 @@ extern "C" int frx_decode_greedy(frx_handle* h, const float* memory, int32_t B, 
                                  int64_t* tokens, const int64_t* forced, void* stream) {
   if (!h) return 1;
   return decode_greedy_impl(h, memory, B, steps, logits, tokens, forced, (cudaStream_t)stream);
+}
+
+extern "C" int frx_decode_greedy_eos(frx_handle* h, const float* memory, int32_t B, int32_t max_steps, float* logits,
+                                     int64_t* tokens, int32_t* lengths, const int64_t* forced, int32_t managed, void* stream) {
+  if (!h) return 1;
+  if (!lengths) return fail(h, "decode_greedy_eos: lengths must not be NULL");
+  return decode_greedy_impl(h, memory, B, max_steps, logits, tokens, forced, (cudaStream_t)stream, managed != 0, lengths);
+}
+
+extern "C" int frx_forward_greedy_eos(frx_handle* h, const float* images, int32_t B, int32_t max_steps, float* logits,
+                                      int64_t* tokens, int32_t* lengths, int32_t managed, void* stream) {
+  if (!h) return 1;
+  if (frx_encode(h, images, B, h->memory_int, stream)) return 1;
+  return frx_decode_greedy_eos(h, h->memory_int, B, max_steps, logits, tokens, lengths, nullptr, managed, stream);
 }
 
 // DecodingManager (postprocessing/postprocessing.py:182-405): upload the per-token rule tables.

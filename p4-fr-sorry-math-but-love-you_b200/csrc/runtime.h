@@ -121,6 +121,7 @@ struct frx_handle {
   float *logits_int = nullptr, *memory_int = nullptr, *images_int = nullptr;
   long long *tokens_int = nullptr, *forced_int = nullptr;
   int* cur_tok = nullptr;
+  int* eos_work = nullptr;       // work counter of the stop-at-<EOS> decode kernel
   void* mem_bf = nullptr;  // bf16 copy of the encoder memory (A operand of the cross K/V GEMM)
   void *kself_bf = nullptr, *vself_bf = nullptr, *kcross_bf = nullptr, *vcross_bf = nullptr;  // bf16 caches
 

@@ -2,12 +2,17 @@
 import torch
 
 
-def decode(model, input, data_loader=None, expected=None, method="greedy", beam_width=3):
+def decode(model, input, data_loader=None, expected=None, method="greedy", beam_width=3, stop_at_eos=False):
     """Same arguments, return value and error behaviour as the reference's
     ``decode``: greedy -> int64 [B, expected.size(1)-1] on the input's device
     (logits -> transpose -> topk(1) over the vocab axis, decoding.py:35-40);
-    beam -> int64 [B, expected.size(-1)-1] on the CPU (decoding.py:42-48)."""
-    if method == "greedy":
+    beam -> int64 [B, expected.size(-1)-1] on the CPU (decoding.py:42-48).
+
+    ``stop_at_eos`` (greedy only; beam search stops at <EOS> already): decode each image only up to its first <EOS>
+    and return <PAD> after it -- the same strings from id_to_string (utils/utils.py:134-164), less decoder work."""
+    if method == "greedy" and stop_at_eos:
+        _, sequence, _ = model.greedy_until_eos(input, expected.size(1) - 1)
+    elif method == "greedy":
         output = model(input=input, expected=expected, is_train=False, teacher_forcing_ratio=0.0)
         decoded_values = output.transpose(1, 2)
         _, sequence = torch.topk(decoded_values, 1, dim=1)

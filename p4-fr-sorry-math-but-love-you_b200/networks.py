@@ -448,6 +448,28 @@ class EfficientSATRN(_FrxModule):
         eng.h.call("frx_decode_greedy", _ptr(memory), b, steps, _ptr(logits), _ptr(tokens), _ptr(f), _stream(dev))
         return logits, tokens
 
+    def greedy_until_eos(self, input, max_steps, forced=None, want_logits=False):
+        """Encode + greedy decode that stops each image at its first <EOS> (frx_decode_greedy_eos): returns
+        (logits | None, tokens [B, max_steps] int64, lengths [B] int32) on the input's device.  Up to lengths[b] the
+        logits and tokens are the full greedy decode's (bitwise); after it tokens are <PAD> and logits rows 0.  With a
+        DecodingManager attached the rows are its masked probabilities and the tokens its picks.  ``forced`` feeds given
+        tokens; row b then stops after the step where forced[b, t] is <EOS>."""
+        b = input.size(0)
+        eng = self.engine(input.device, b, max_steps)
+        x = input.detach().float().contiguous()
+        dev = x.device
+        managed = self.decoder.manager is not None
+        if managed:
+            self._attach_manager(eng)
+        memory = self.encode(x)
+        logits = torch.empty(b, max_steps, self._dims["num_classes"], device=dev) if want_logits else None
+        tokens = torch.empty(b, max_steps, dtype=torch.int64, device=dev)
+        lengths = torch.empty(b, dtype=torch.int32, device=dev)
+        f = forced.to(device=dev, dtype=torch.int64).contiguous() if forced is not None else None
+        eng.h.call("frx_decode_greedy_eos", _ptr(memory), b, max_steps, _ptr(logits), _ptr(tokens), _ptr(lengths), _ptr(f),
+                   int(managed), _stream(dev))
+        return logits, tokens, lengths
+
     def greedy_host(self, images_host, steps, tokens_host=None, logits_host=None):
         """End-to-end call with HOST buffers (frx_forward_greedy_host): H2D of the
         images, encode, decode, D2H of the tokens; returns the host token tensor."""
