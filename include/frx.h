@@ -250,7 +250,7 @@ int frx_read_prof(frx_handle* h, int64_t* out16);
  *                                                                BatchNorm batch statistics)
  *   loss = CrossEntropyLoss(ignore_index=PAD)(output.transpose(1, 2), expected[:, 1:])   (:82-86, EfficientSATRN.py:690-692)
  *   loss.backward(); clip_grad_norm_(params, max_grad_norm); AdamW.step()                (:92-98, utils/utils.py:91-92)
- * fp32 like the reference (no autocast); dropout is not applied (p = 0).
+ * fp32 like the reference (no autocast).  Dropout is off unless frx_train_set_dropout enables it.
  *
  * frx_train_create      copies the loaded parameters into the training state (one flat fp32 buffer in kernel layouts, a
  *                       parallel gradient buffer, Adam moments, BatchNorm running statistics) and sizes the activation
@@ -300,6 +300,19 @@ int64_t frx_train_step_count(const frx_handle* h);
  * would see): copies the named buffer to dst (host or device, capacity floats) and returns its length; dst = NULL only
  * returns the length; -1 = unknown name.  Names: "dec<l>.d_linear0", "dec<l>.d_linear1", "dec<l>.d_ffn_out", ... */
 int64_t frx_train_read_tap(frx_handle* h, const char* name, float* dst, int64_t capacity);
+/* Dropout in the training pass (off after frx_train_create; p = p_ffn = 0 turns it off again).  p is the rate of the
+ * reference's sites (FLAGS.dropout_rate): the 2-D PE output, the attention probabilities and the MHA outputs of every
+ * encoder and decoder layer, the decoder input; p_ffn the rate after each ReLU of the decoder feed-forward blocks (0.1 in
+ * the reference whatever the flag says).  Masks come from Philox4x32-10 with key = seed (low word, high word) and counter
+ * (element index / 4, site + 16 * layer, step, rank), element index in the reference's layout of the site; step counts
+ * the forward passes since frx_train_create, rank is the data-parallel rank.  An element is kept iff its word is
+ * >= min(2^32 - 1, floor(p * 2^32)) (p as this float, computed in double); kept values are multiplied by
+ * 1.0f / (1.0f - p).  The backward pass regenerates the masks of the forward pass it continues.  Rates outside [0, 1)
+ * and a handle without training state are rejected.  Inference never applies dropout. */
+int frx_train_set_dropout(frx_handle* h, float p, float p_ffn, uint64_t seed, int32_t rank);
+/* Test hook: Philox4x32-10 of one counter and key, computed on the GPU by the function the dropout kernels use
+ * (synchronous, host in and out). */
+int frx_philox4x32(const uint32_t ctr[4], const uint32_t key[2], uint32_t out[4]);
 
 #ifdef __cplusplus
 }

@@ -17,7 +17,7 @@ SYMBOLS = [
     "frx_train_create", "frx_train_destroy", "frx_train_param_count", "frx_train_fwd_bwd", "frx_train_grad_buffer",
     "frx_train_set_bucket_callback", "frx_train_apply", "frx_train_export", "frx_train_read_grad", "frx_train_step_count", "frx_train_read_tap",
     "frx_train_forward", "frx_train_backward", "frx_train_import", "frx_ensemble_decode", "frx_preprocess_u8", "frx_train_apply_dual",
-    "frx_decode_greedy_eos", "frx_forward_greedy_eos",
+    "frx_decode_greedy_eos", "frx_forward_greedy_eos", "frx_train_set_dropout", "frx_philox4x32",
 ]
 
 BUCKET_CALLBACK = ctypes.CFUNCTYPE(None, ctypes.c_void_p, ctypes.c_int64, ctypes.c_int64)
@@ -104,6 +104,9 @@ def load_library():
     lib.frx_train_read_tap.restype = i64
     lib.frx_train_step_count.argtypes = [vp]
     lib.frx_train_step_count.restype = i64
+    lib.frx_train_set_dropout.argtypes = [vp, f32, f32, ctypes.c_uint64, i32]
+    u32x = ctypes.POINTER(ctypes.c_uint32)
+    lib.frx_philox4x32.argtypes = [u32x, u32x, u32x]
     _LIB = lib
     return lib
 

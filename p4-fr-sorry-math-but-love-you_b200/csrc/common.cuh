@@ -117,6 +117,37 @@ struct GemmP {
   int splitk, k_chunk; // set by the launcher
 };
 
+// Philox4x32-10 (Random123; the generator of curand_Philox4x32_10): counter c, key k -> four 32-bit words
+__host__ __device__ __forceinline__ uint4 philox4x32_10(uint4 c, uint2 k) {
+#pragma unroll
+  for (int r = 0; r < 10; ++r) {
+    const uint64_t p0 = (uint64_t)0xD2511F53u * c.x, p1 = (uint64_t)0xCD9E8D57u * c.z;
+    c = make_uint4((uint32_t)(p1 >> 32) ^ c.y ^ k.x, (uint32_t)p1, (uint32_t)(p0 >> 32) ^ c.w ^ k.y, (uint32_t)p0);
+    k.x += 0x9E3779B9u;
+    k.y += 0xBB67AE85u;
+  }
+  return c;
+}
+
+// One dropout site of the training step.  Element e (its index in the site's logical layout) is kept iff word e % 4 of
+// philox4x32_10((e / 4, site, step, rank), (seed_lo, seed_hi)) is >= thresh; kept values are multiplied by scale, dropped
+// ones are 0.  step is read from device memory (*step - back), so a CUDA graph of the pass draws new masks on every replay:
+// the forward kernels read the counter with back = 0, the backward kernels (after the forward has advanced it) with 1.
+struct DropP {
+  const uint32_t* step;   // nullptr: the site is off
+  uint32_t back;
+  uint32_t site, rank;
+  uint32_t key_lo, key_hi;
+  uint32_t thresh;
+  float scale;
+};
+__device__ __forceinline__ float drop_factor(const DropP& d, long long e) {
+  const uint4 r = philox4x32_10(make_uint4((uint32_t)(e >> 2), d.site, *d.step - d.back, d.rank), make_uint2(d.key_lo, d.key_hi));
+  const int w = (int)(e & 3);
+  const uint32_t u = w == 0 ? r.x : w == 1 ? r.y : w == 2 ? r.z : r.w;
+  return u >= d.thresh ? d.scale : 0.f;
+}
+
 struct DwP {
   const float* in;     // NHWC [B,H,W,C]
   const float* w;      // [9][C]

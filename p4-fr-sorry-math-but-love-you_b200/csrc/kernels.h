@@ -23,6 +23,9 @@ void launch_layernorm_f32(const float* x, const float* res, const float* gamma, 
 void launch_enc_attn_f32(const float* qkv, float* out, int B, int S, int D, int heads, cudaStream_t st);
 void launch_dec_gemm_f32(const DecGemmP& p, cudaStream_t st);
 void launch_dec_attn_f32(const AttnP& p, int head_dim, cudaStream_t st);
+// training-step variants with attention dropout on the probabilities (common.cuh DropP)
+void launch_enc_attn_f32_drop(const float* qkv, float* out, int B, int S, int D, int heads, const DropP& drop, cudaStream_t st);
+void launch_dec_attn_f32_drop(const AttnP& p, int head_dim, const DropP& drop, cudaStream_t st);
 void launch_fill_i32(int* p, int v, int n, cudaStream_t st);
 void launch_dec_embed_f32(const int* tok, const long long* tok64, int fixed_token, const float* emb,
                           const float* pe, int pos, const int* pos_arr, int pos_mod, float scale, float* x,

@@ -1161,7 +1161,24 @@ FRX_DEC_NAME(dec_cluster_bf16_kernel)(const DecClusterP p) {
       bool busy = false;
 #pragma unroll
       for (int i = 0; i < NIMG; ++i) busy = busy || er.img[i] >= 0;
-      if (!busy) break;   // the same decision in every CTA of the cluster
+      if (!busy) {   // the same decision in every CTA of the cluster
+        if constexpr (EARLY_PRIME) {
+          // a row that finished in this step has K/V blocks in flight, requested for a next step that will not come: they
+          // must land before the CTA exits, or a bulk copy completes into the shared memory of the next CTA on this SM
+          if (self_primed && er.done[wimg]) {
+            const int primed_n = er.left[wimg];
+#pragma unroll
+            for (int d = 0; d < KVD; ++d) {
+              if (32 * d < primed_n) {
+                mbar_wait(kvbar + 8u * d, (kvphase >> d) & 1u);
+                kvphase ^= 1u << d;
+              }
+            }
+            __syncwarp();
+          }
+        }
+        break;
+      }
     }
   }
   cl.sync();  // nobody exits while a peer's stores to it may still be in flight

@@ -660,10 +660,12 @@ void launch_layernorm_bf16out(const float* x, const float* res, const float* gam
 // 8. Encoder self-attention (:164-172,:198-228): one CTA per (image, head);
 //    S tokens x HD=64; scores divided by sqrt(heads*HD).
 // ===========================================================================
-template <typename OutT>
+// DROP (training step only): attention dropout on the probabilities [B, heads, S, S] -- the softmax sum is taken over the
+// undropped probabilities, P.M.scale multiplies V.
+template <typename OutT, bool DROP = false>
 __global__ void __launch_bounds__(128) enc_attn_f32_kernel(const float* __restrict__ qkv,  // [B*S, 3*D]
                                                            OutT* __restrict__ out,        // [B*S, D]
-                                                           int S, int D, int heads, float temperature) {
+                                                           int S, int D, int heads, float temperature, DropP drop) {
   extern __shared__ float sm[];
   const int HD = D / heads;  // 64
   const int LDS_ = HD + 1;
@@ -700,10 +702,16 @@ __global__ void __launch_bounds__(128) enc_attn_f32_kernel(const float* __restri
       sum += e;
     }
     sum = warp_sum(sum);
+    if constexpr (DROP) {
+      for (int j = lane; j < S; j += 32) Pw[j] *= drop_factor(drop, ((long long)blockIdx.x * S + i) * S + j) != 0.f ? 1.f : 0.f;
+    }
     __syncwarp();
     for (int c = lane; c < HD; c += 32) {
       float acc = 0.f;
-      for (int j = 0; j < S; ++j) acc = fmaf(Pw[j] / sum, V[j * LDS_ + c], acc);
+      for (int j = 0; j < S; ++j) {
+        if constexpr (DROP) acc = fmaf(__fmul_rn(Pw[j] / sum, drop.scale), V[j * LDS_ + c], acc);
+        else acc = fmaf(Pw[j] / sum, V[j * LDS_ + c], acc);
+      }
       store_as(out + ((long long)b * S + i) * D + hh * HD + c, acc);
     }
     __syncwarp();
@@ -716,10 +724,16 @@ static void enc_attn_launch(const float* qkv, OutT* out, int B, int S, int D, in
   size_t smem = (size_t)(3 * S * (HD + 1) + 4 * S) * sizeof(float);
   static SmemOptIn opt;
   opt.ensure(enc_attn_f32_kernel<OutT>, smem);
-  enc_attn_f32_kernel<OutT><<<B * heads, 128, smem, st>>>(qkv, out, S, D, heads, sqrtf((float)D));
+  enc_attn_f32_kernel<OutT><<<B * heads, 128, smem, st>>>(qkv, out, S, D, heads, sqrtf((float)D), DropP{});
 }
 void launch_enc_attn_f32(const float* qkv, float* out, int B, int S, int D, int heads, cudaStream_t st) {
   enc_attn_launch<float>(qkv, out, B, S, D, heads, st);
+}
+void launch_enc_attn_f32_drop(const float* qkv, float* out, int B, int S, int D, int heads, const DropP& drop, cudaStream_t st) {
+  const size_t smem = (size_t)(3 * S * (D / heads + 1) + 4 * S) * sizeof(float);
+  static SmemOptIn opt;
+  opt.ensure(enc_attn_f32_kernel<float, true>, smem);
+  enc_attn_f32_kernel<float, true><<<B * heads, 128, smem, st>>>(qkv, out, S, D, heads, sqrtf((float)D), drop);
 }
 void launch_enc_attn_bf16out(const float* qkv, eh_t* out, int B, int S, int D, int heads, cudaStream_t st) {
   enc_attn_launch<eh_t>(qkv, out, B, S, D, heads, st);
@@ -841,8 +855,10 @@ void launch_dec_gemm_f32(const DecGemmP& p, cudaStream_t st) {
 //     one warp per (query row, head), HD = 32 -> lane = channel for P.V.
 //     Implements :164-172 on the recurrence of SURVEY App. A.4.
 // ===========================================================================
-template <int HD>
-__global__ void __launch_bounds__(256) dec_attn_f32_kernel(const AttnP p) {
+// DROP (training step only): attention dropout on the probabilities, logical layout [images, heads, q_per_img,
+// rows_per_img] (teacher forcing: [B, H, L, L] / [B, H, L, S]); the softmax sum is over the undropped probabilities.
+template <int HD, bool DROP = false>
+__global__ void __launch_bounds__(256) dec_attn_f32_kernel(const AttnP p, DropP drop) {
   extern __shared__ float sm[];  // [8 warps][max_keys]
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const int gw = blockIdx.x * 8 + warp;
@@ -892,6 +908,10 @@ __global__ void __launch_bounds__(256) dec_attn_f32_kernel(const AttnP p) {
     sum += e;
   }
   sum = warp_sum(sum);
+  if constexpr (DROP) {
+    const long long row = ((long long)img * p.heads + hh) * p.q_per_img + m % p.q_per_img;
+    for (int j = lane; j < nk; j += 32) sc[j] *= drop_factor(drop, row * p.rows_per_img + j) != 0.f ? 1.f : 0.f;
+  }
   __syncwarp();
   float acc[PER];
 #pragma unroll
@@ -901,6 +921,7 @@ __global__ void __launch_bounds__(256) dec_attn_f32_kernel(const AttnP p) {
     if (j < nh) vp = vbase + (long long)(chain ? __ldg(chain + j) : j) * p.D;
     else vp = p.cur_v + (long long)m * p.ld_cur + hh * HD;
     float pj = sc[j] / sum;
+    if constexpr (DROP) pj = __fmul_rn(pj, drop.scale);
 #pragma unroll
     for (int i = 0; i < PER; ++i) acc[i] = fmaf(pj, __ldg(vp + i * 32 + lane), acc[i]);
   }
@@ -911,8 +932,14 @@ __global__ void __launch_bounds__(256) dec_attn_f32_kernel(const AttnP p) {
 void launch_dec_attn_f32(const AttnP& p, int head_dim, cudaStream_t st) {
   int warps = p.M * p.heads;
   size_t smem = (size_t)8 * (p.rows_per_img + 1) * sizeof(float);
-  if (head_dim == 32) dec_attn_f32_kernel<32><<<(warps + 7) / 8, 256, smem, st>>>(p);
-  else dec_attn_f32_kernel<64><<<(warps + 7) / 8, 256, smem, st>>>(p);
+  if (head_dim == 32) dec_attn_f32_kernel<32><<<(warps + 7) / 8, 256, smem, st>>>(p, DropP{});
+  else dec_attn_f32_kernel<64><<<(warps + 7) / 8, 256, smem, st>>>(p, DropP{});
+}
+void launch_dec_attn_f32_drop(const AttnP& p, int head_dim, const DropP& drop, cudaStream_t st) {
+  const int warps = p.M * p.heads;
+  const size_t smem = (size_t)8 * (p.rows_per_img + 1) * sizeof(float);
+  if (head_dim == 32) dec_attn_f32_kernel<32, true><<<(warps + 7) / 8, 256, smem, st>>>(p, drop);
+  else dec_attn_f32_kernel<64, true><<<(warps + 7) / 8, 256, smem, st>>>(p, drop);
 }
 
 // ===========================================================================

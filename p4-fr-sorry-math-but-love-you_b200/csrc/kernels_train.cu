@@ -57,6 +57,31 @@ void launch_axpy(float* y, const float* x, float a, long long n, int accumulate,
   if (n > 0) axpy_kernel<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(y, x, a, n, accumulate);
 }
 
+// dropout: y = x * M * scale (+ add).  Element i of the row-major buffer has the logical index i, or with S > 0 the buffer
+// is NHWC [B, S, C] and the logical layout NCHW [B, C, S].  In place (y == x) is allowed.
+__global__ void __launch_bounds__(256) dropout_kernel(const float* x, const float* __restrict__ add, float* y, long long n, const DropP d, int S,
+                                                      int C) {
+  long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= n) return;
+  long long e = i;
+  if (S > 0) {
+    const long long b = i / ((long long)S * C);
+    const int c = (int)(i % C), q = (int)((i / C) % S);
+    e = (b * C + c) * S + q;
+  }
+  const float v = __fmul_rn(x[i], drop_factor(d, e));
+  y[i] = add ? __fadd_rn(v, add[i]) : v;
+}
+void launch_dropout(const float* x, const float* add, float* y, long long n, const DropP& d, int S, int C, cudaStream_t st) {
+  if (n > 0) dropout_kernel<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(x, add, y, n, d, S, C);
+}
+// the dropout step counter: *ctr += v (one thread)
+__global__ void counter_add_kernel(uint32_t* ctr, uint32_t v) { *ctr += v; }
+void launch_counter_add(uint32_t* ctr, uint32_t v, cudaStream_t st) { counter_add_kernel<<<1, 1, 0, st>>>(ctr, v); }
+// philox4x32_10 of one counter / key (the test hook frx_philox4x32)
+__global__ void philox_probe_kernel(uint4* io) { io[0] = philox4x32_10(io[0], make_uint2(io[1].x, io[1].y)); }
+void launch_philox_probe(uint4* io, cudaStream_t st) { philox_probe_kernel<<<1, 1, 0, st>>>(io); }
+
 // out = act(in); dgrad variant: out = dout * act'(pre)
 __global__ void __launch_bounds__(256) act_fwd_kernel(const float* __restrict__ in, float* __restrict__ out, int act, long long n) {
   long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
@@ -532,19 +557,23 @@ void launch_spatial_scale(const float* x, const float* g, const float* add, floa
   spatial_scale_kernel<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(x, g, add, out, S, C, n);
 }
 
-// adaptive 2-D PE apply: out = x + g[b][c] * peh[row][c] + g[b][C + c] * pew[col][c]
+// adaptive 2-D PE apply: out = x + g[b][c] * peh[row][c] + g[b][C + c] * pew[col][c]; with drop.step, dropout on out with
+// the mask of the reference's NCHW layout [B, C, h, w]
 __global__ void __launch_bounds__(256) pe2d_apply_kernel(const float* __restrict__ x, const float* __restrict__ g, const float* __restrict__ peh,
-                                                         const float* __restrict__ pew, float* __restrict__ out, int h, int w, int C, long long n) {
+                                                         const float* __restrict__ pew, float* __restrict__ out, int h, int w, int C, long long n,
+                                                         const DropP drop) {
   long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= n) return;
   const int c = (int)(i % C);
   const int q = (int)((i / C) % (h * w));
   const long long b = i / ((long long)h * w * C);
-  out[i] = x[i] + g[b * 2 * C + c] * __ldg(peh + (q / w) * C + c) + g[b * 2 * C + C + c] * __ldg(pew + (q % w) * C + c);
+  const float v = x[i] + g[b * 2 * C + c] * __ldg(peh + (q / w) * C + c) + g[b * 2 * C + C + c] * __ldg(pew + (q % w) * C + c);
+  out[i] = drop.step ? __fmul_rn(v, drop_factor(drop, (b * C + c) * h * w + q)) : v;
 }
-void launch_pe2d_apply(const float* x, const float* g, const float* peh, const float* pew, float* out, int B, int h, int w, int C, cudaStream_t st) {
+void launch_pe2d_apply(const float* x, const float* g, const float* peh, const float* pew, float* out, int B, int h, int w, int C,
+                       const DropP& drop, cudaStream_t st) {
   const long long n = (long long)B * h * w * C;
-  pe2d_apply_kernel<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(x, g, peh, pew, out, h, w, C, n);
+  pe2d_apply_kernel<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(x, g, peh, pew, out, h, w, C, n, drop);
 }
 // dg[b][c] = sum_q dout * peh[row][c];  dg[b][C + c] = sum_q dout * pew[col][c]
 __global__ void __launch_bounds__(256) pe2d_bwd_gate_kernel(const float* __restrict__ dout, const float* __restrict__ peh, const float* __restrict__ pew,
@@ -695,12 +724,16 @@ __global__ void __launch_bounds__(256) attn_bwd_kernel(const AttnBwdP p) {
     int cnt = 0;
     for (int j = lane; j < Lk; j += 32, ++cnt) {
       const float pj = pw[j] * inv;
+      // dropout on the probabilities: the forward multiplied V by P.M.s, so dP = (dout . v_j) M.s and dv_j += P M.s dout
+      const float mj = p.drop.step ? drop_factor(p.drop, (((long long)b * p.heads + hh) * Lq + i) * Lk + j) : 1.f;
       float dp = 0.f;
       for (int d = 0; d < HD; ++d) dp = fmaf(dop[d], sv[j * (HD + 1) + d], dp);
+      if (p.drop.step) dp = __fmul_rn(dp, mj);
       dpj[cnt] = dp;
       delta = fmaf(pj, dp, delta);
       // dv_j += p_j * dout
-      for (int d = 0; d < HD; ++d) atomicAdd(&sdv[j * (HD + 1) + d], pj * dop[d]);
+      const float pv = p.drop.step ? __fmul_rn(pj, mj) : pj;
+      for (int d = 0; d < HD; ++d) atomicAdd(&sdv[j * (HD + 1) + d], pv * dop[d]);
     }
     delta = warp_sum(delta);
     cnt = 0;
@@ -791,16 +824,20 @@ __global__ void __launch_bounds__(256) attn_bwd_split_kernel(const AttnBwdP p) {
     sum = warp_sum(sum);
     const float inv = 1.f / sum;
     float delta = 0.f;
+    const long long erow = (((long long)b * p.heads + hh) * Lq + i) * Lk;   // dropout mask row (logical [B, heads, Lq, Lk])
     for (int j = lane; j < Lk; j += 32) {
       const float pj = pw[j] * inv;
       float dp = 0.f;
       for (int d = 0; d < HD; ++d) dp = fmaf(dop[d], sv[j * (HD + 1) + d], dp);
+      if (p.drop.step) dp = __fmul_rn(dp, drop_factor(p.drop, erow + j));   // dP = (dO V^T) M.s
       pw[j] = pj;
       dsw[j] = dp;
       delta = fmaf(pj, dp, delta);
     }
     delta = warp_sum(delta);
     for (int j = lane; j < Lk; j += 32) dsw[j] = pw[j] * (dsw[j] - delta) * inv_t;
+    if (p.drop.step)   // dV below takes the probabilities the forward multiplied V by: P.M.s
+      for (int j = lane; j < Lk; j += 32) pw[j] = __fmul_rn(pw[j], drop_factor(p.drop, erow + j));
     __syncwarp();
     for (int d = lane; d < HD; d += 32) {   // dq_i = sum_j ds_j k_j
       float acc = 0.f;

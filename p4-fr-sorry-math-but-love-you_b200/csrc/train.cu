@@ -5,8 +5,7 @@
 //                                                                        networks/EfficientSATRN.py:488-495, :697-706)
 //   loss = CrossEntropyLoss(ignore_index=PAD)(output.transpose(1, 2), expected[:, 1:])     (:82-86, :690-692)
 //   loss.backward(); clip_grad_norm_(params, max_grad_norm); AdamW.step()                  (:92-98, utils/utils.py:91-92)
-// fp32 throughout, like the reference (no autocast).  Dropout is not applied (p = 0: the reference draws its masks from
-// torch's global RNG; parity runs set every nn.Dropout to 0).  Data-parallel training: frx_train_fwd_bwd leaves the
+// fp32 throughout, like the reference (no autocast).  Data-parallel training: frx_train_fwd_bwd leaves the
 // gradients in ONE flat buffer (frx_train_grad_buffer) that the host all-reduces with NCCL -- per bucket, as soon as
 // the backward pass has enqueued the kernels that produce it (frx_train_set_bucket_callback) -- before
 // frx_train_apply clips and applies AdamW.
@@ -14,6 +13,16 @@
 // Parameters live in one flat fp32 buffer in the layouts the kernels consume (conv [O][kh][kw][I], depthwise [9][C],
 // q|k|v concatenated); gradients, Adam moments are parallel buffers, so the optimiser, the norm and the all-reduce are
 // layout-agnostic.  frx_train_export / frx_train_read_grad convert back to the reference's state_dict layout.
+//
+// Dropout (opt-in, frx_train_set_dropout; off by default, and then the pass is the one without it) at the reference's
+// sites: 0 the 2-D PE output; per encoder layer 1 the attention probabilities, 2 the MHA output before the residual add;
+// 3 the decoder input; per decoder layer 4 / 5 self-attention probabilities / output, 6 / 7 cross-attention probabilities
+// / output (rate p), 8 / 9 after each feed-forward ReLU (rate p_ffn).  The masks come from Philox4x32-10 (common.cuh
+// philox4x32_10 / DropP) with counter (element index / 4, site + 16 * layer, step, rank) and the 64-bit seed as key, over
+// the reference's logical layout of each site.  They are never stored: the backward kernels regenerate them.  step counts
+// the forward passes since frx_train_create; it lives in device memory and the pass advances it itself, so a replay of the
+// pass's CUDA graph draws new masks.
+#include <algorithm>
 #include <cmath>
 #include <cstdarg>
 #include <cstdio>
@@ -90,8 +99,9 @@ struct DWS { const float* x; float *z, *y, *stat; int B, H, W, C, OH, OW, stride
 struct SES { const float* y2; float *s, *p1, *hh, *p2, *g, *y3; int B, S, C, R; };
 struct BlockSave { CB c1, c2; DWS dw; SES se; const float* x_in; float* y_out; };
 struct LNS { const float* x; float* y; float* stat; int M, C; size_t g, b; };
-struct EncSave { LNS ln1, ln2; float *qkv, *att, *pre2, *scr; CB c0, c1; DWS dw; const float* x_in; };
-struct DecSave { const float* x_in; float *qkv, *att, *pre1, *q2, *kv, *catt, *pre2, *f0, *f1, *pre3; LNS ln1, ln2, ln3; };
+// o / o1 / o2: out_linear's result before dropout and the residual add (only with dropout on)
+struct EncSave { LNS ln1, ln2; float *qkv, *att, *pre2, *scr; CB c0, c1; DWS dw; const float* x_in; float* o; };
+struct DecSave { const float* x_in; float *qkv, *att, *pre1, *q2, *kv, *catt, *pre2, *f0, *f1, *pre3; LNS ln1, ln2, ln3; float *o1, *o2; };
 
 // what the backward pass needs from the forward pass of the same call (or of the preceding frx_train_forward call)
 struct Tape {
@@ -161,6 +171,16 @@ struct TrainState {
   unsigned long long graph_clock = 0;
   float* img_stage = nullptr;
   long long* exp_stage = nullptr;
+  // dropout (frx_train_set_dropout)
+  float drop_p = 0.f, drop_pffn = 0.f;
+  uint64_t drop_seed = 0;
+  int drop_rank = 0;
+  uint32_t* drop_ctr = nullptr;   // device: forward passes so far, advanced by the passes that run with dropout
+  uint32_t drop_pending = 0;      // forward passes without dropout not yet added to *drop_ctr
+  float graph_p = 0.f, graph_pffn = 0.f;   // the setting the cached graphs with dropout were captured with
+  uint64_t graph_seed = 0;
+  int graph_rank = 0;
+  bool drop_on() const { return drop_p > 0.f || drop_pffn > 0.f; }
 };
 
 struct Ctx {   // one training call
@@ -553,6 +573,45 @@ int ln_bwd(Ctx& c, const LNS& r, const float* dy, float** dx_out) {
 
 void tap(Ctx& c, const std::string& name, const float* p, size_t n) { c.T->taps[name] = {p, n}; }
 
+// dropout site `site` of layer `layer` (ffn: rate p_ffn, else p); back = 1 in the backward pass, which runs after the forward
+// pass has advanced the step counter.  step == nullptr when the site's rate is 0.
+DropP drop_site(const TrainState* T, int site, int layer, bool ffn, int back) {
+  DropP d{};
+  const float p = ffn ? T->drop_pffn : T->drop_p;
+  if (p <= 0.f) return d;
+  d.step = T->drop_ctr;
+  d.back = (uint32_t)back;
+  d.site = (uint32_t)(site + 16 * layer);
+  d.rank = (uint32_t)T->drop_rank;
+  d.key_lo = (uint32_t)T->drop_seed;
+  d.key_hi = (uint32_t)(T->drop_seed >> 32);
+  d.thresh = (uint32_t)std::min(4294967295.0, std::floor((double)p * 4294967296.0));
+  d.scale = 1.0f / (1.0f - p);
+  return d;
+}
+
+// out_linear of an attention block: y = dropout(x W^T + b) + res, or with the site off the GEMM with the residual in its
+// epilogue.  o: tape buffer for the undropped GEMM result.
+int attn_out_fwd(Ctx& c, const float* x, long long M, int N, size_t w, size_t b, const float* res, float* y, float** o, const DropP& d) {
+  frx_handle* h = c.h;
+  if (!d.step) return lin_fwd(c, x, M, N, w, b, true, N, y, N, ACT_NONE, res);
+  WALLOC(*o, M * N);
+  if (lin_fwd(c, x, M, N, w, b, true, N, *o, N, ACT_NONE, nullptr)) return 1;
+  launch_dropout(*o, res, y, M * N, d, 0, 0, c.st); TKL();
+  return 0;
+}
+// gradient of out_linear's output under dropout: dy * M * s into a fresh buffer (dy itself when the site is off)
+int drop_bwd(Ctx& c, const float* dy, long long n, const DropP& d, const float** out) {
+  frx_handle* h = c.h;
+  *out = dy;
+  if (!d.step) return 0;
+  float* m;
+  WALLOC(m, n);
+  launch_dropout(dy, nullptr, m, n, d, 0, 0, c.st); TKL();
+  *out = m;
+  return 0;
+}
+
 void bucket_done(Ctx& c, int idx) {
   if (c.T->bucket_cb && idx < (int)c.T->buckets.size() && c.T->buckets[idx].second > 0)
     c.T->bucket_cb(c.T->bucket_ctx, (int64_t)c.T->buckets[idx].first, (int64_t)c.T->buckets[idx].second);
@@ -662,7 +721,7 @@ int fwd_bwd(Ctx& c, const float* images, const long long* expected, float* loss_
   launch_act_fwd(tp.pe_hp, tp.pe_h, ACT_RELU, (long long)B * C / 2, c.st); TKL();
   if (lin_fwd(c, tp.pe_h, B, C / 2, T->pe_w1, T->pe_b1, true, 2 * C, tp.pe_gp, 2 * C, ACT_NONE, nullptr)) return 1;
   launch_act_fwd(tp.pe_gp, tp.pe_g, ACT_SIGMOID, (long long)B * 2 * C, c.st); TKL();
-  launch_pe2d_apply(tp.trunk_out, tp.pe_g, peh, pew, tp.pe_out, B, tp.H, tp.W, C, c.st); TKL();
+  launch_pe2d_apply(tp.trunk_out, tp.pe_g, peh, pew, tp.pe_out, B, tp.H, tp.W, C, drop_site(T, 0, 0, false, 0), c.st); TKL();
   // ---- encoder layers (:259-281) ----
   tp.es.assign(T->enc.size(), EncSave{});
   const float* xe = tp.pe_out;
@@ -675,8 +734,11 @@ int fwd_bwd(Ctx& c, const float* images, const long long* expected, float* loss_
     if (ln_fwd(c, s.ln1)) return 1;
     WALLOC(s.qkv, (size_t)Me * 3 * C); WALLOC(s.att, (size_t)Me * C); WALLOC(s.pre2, (size_t)Me * C); WALLOC(s.scr, (size_t)Me * C);
     if (lin_fwd(c, s.ln1.y, Me, C, Lw.w_qkv, Lw.b_qkv, true, 3 * C, s.qkv, 3 * C, ACT_NONE, nullptr)) return 1;
-    launch_enc_attn_f32(s.qkv, s.att, B, S, C, cf.enc_heads, c.st); TKL();
-    if (lin_fwd(c, s.att, Me, C, Lw.w_o, Lw.b_o, true, C, s.pre2, C, ACT_NONE, xe)) return 1;
+    const DropP dpa = drop_site(T, 1, (int)i, false, 0);
+    if (dpa.step) launch_enc_attn_f32_drop(s.qkv, s.att, B, S, C, cf.enc_heads, dpa, c.st);
+    else launch_enc_attn_f32(s.qkv, s.att, B, S, C, cf.enc_heads, c.st);
+    TKL();
+    if (attn_out_fwd(c, s.att, Me, C, Lw.w_o, Lw.b_o, xe, s.pre2, &s.o, drop_site(T, 2, (int)i, false, 0))) return 1;
     s.ln2 = LNS{s.pre2, nullptr, nullptr, Me, C, Lw.ln_g, Lw.ln_b};
     if (ln_fwd(c, s.ln2)) return 1;
     launch_scramble(s.ln2.y, s.scr, B, S, C, 0, c.st); TKL();
@@ -700,6 +762,7 @@ int fwd_bwd(Ctx& c, const float* images, const long long* expected, float* loss_
   float* x0;
   WALLOC(x0, (size_t)Md * D);
   launch_dec_embed_f32(nullptr, tp.text, 0, T->P + T->emb, h->arena + h->pe1d, 0, nullptr, L, temp, x0, Md, D, c.st); TKL();
+  if (const DropP d = drop_site(T, 3, 0, false, 0); d.step) { launch_dropout(x0, nullptr, x0, (long long)Md * D, d, 0, 0, c.st); TKL(); }
   tp.ds.assign(T->dec.size(), DecSave{});
   tp.xd = x0;
   for (size_t l = 0; l < T->dec.size(); ++l) {
@@ -714,9 +777,12 @@ int fwd_bwd(Ctx& c, const float* images, const long long* expected, float* loss_
       AttnP a{};
       a.q = s.qkv; a.ldq = 3 * D; a.kcache = s.qkv + D; a.vcache = s.qkv + 2 * D; a.rows_per_img = L; a.D = 3 * D;
       a.causal_L = L; a.key_mask = tp.mask; a.q_per_img = L; a.temperature = temp; a.out = s.att; a.ldo = D; a.M = Md; a.heads = heads;
-      launch_dec_attn_f32(a, HD, c.st); TKL();
+      const DropP d = drop_site(T, 4, (int)l, false, 0);
+      if (d.step) launch_dec_attn_f32_drop(a, HD, d, c.st);
+      else launch_dec_attn_f32(a, HD, c.st);
+      TKL();
     }
-    if (lin_fwd(c, s.att, Md, D, Wl.w_so, Wl.b_so, true, D, s.pre1, D, ACT_NONE, tp.xd)) return 1;
+    if (attn_out_fwd(c, s.att, Md, D, Wl.w_so, Wl.b_so, tp.xd, s.pre1, &s.o1, drop_site(T, 5, (int)l, false, 0))) return 1;
     s.ln1 = LNS{s.pre1, nullptr, nullptr, Md, D, Wl.ln1_g, Wl.ln1_b};
     if (ln_fwd(c, s.ln1)) return 1;
     if (lin_fwd(c, s.ln1.y, Md, D, Wl.w_cq, Wl.b_cq, true, D, s.q2, D, ACT_NONE, nullptr)) return 1;
@@ -725,13 +791,19 @@ int fwd_bwd(Ctx& c, const float* images, const long long* expected, float* loss_
       AttnP a{};
       a.q = s.q2; a.ldq = D; a.kcache = s.kv; a.vcache = s.kv + D; a.rows_per_img = S; a.D = 2 * D; a.n_hist = S; a.q_per_img = L;
       a.temperature = temp; a.out = s.catt; a.ldo = D; a.M = Md; a.heads = heads;
-      launch_dec_attn_f32(a, HD, c.st); TKL();
+      const DropP d = drop_site(T, 6, (int)l, false, 0);
+      if (d.step) launch_dec_attn_f32_drop(a, HD, d, c.st);
+      else launch_dec_attn_f32(a, HD, c.st);
+      TKL();
     }
-    if (lin_fwd(c, s.catt, Md, D, Wl.w_co, Wl.b_co, true, D, s.pre2, D, ACT_NONE, s.ln1.y)) return 1;
+    if (attn_out_fwd(c, s.catt, Md, D, Wl.w_co, Wl.b_co, s.ln1.y, s.pre2, &s.o2, drop_site(T, 7, (int)l, false, 0))) return 1;
     s.ln2 = LNS{s.pre2, nullptr, nullptr, Md, D, Wl.ln2_g, Wl.ln2_b};
     if (ln_fwd(c, s.ln2)) return 1;
+    // feed-forward dropout after each ReLU, in place: f0 / f1 hold the dropped activations
     if (lin_fwd(c, s.ln2.y, Md, D, Wl.w_f0, Wl.b_f0, true, FF, s.f0, FF, ACT_RELU, nullptr)) return 1;
+    if (const DropP d = drop_site(T, 8, (int)l, true, 0); d.step) { launch_dropout(s.f0, nullptr, s.f0, (long long)Md * FF, d, 0, 0, c.st); TKL(); }
     if (lin_fwd(c, s.f0, Md, FF, Wl.w_f1, Wl.b_f1, true, D, s.f1, D, ACT_RELU, nullptr)) return 1;
+    if (const DropP d = drop_site(T, 9, (int)l, true, 0); d.step) { launch_dropout(s.f1, nullptr, s.f1, (long long)Md * D, d, 0, 0, c.st); TKL(); }
     launch_axpy(s.pre3, s.f1, 1.f, (long long)Md * D, 0, c.st); TKL();
     launch_axpy(s.pre3, s.ln2.y, 1.f, (long long)Md * D, 1, c.st); TKL();
     s.ln3 = LNS{s.pre3, nullptr, nullptr, Md, D, Wl.ln3_g, Wl.ln3_b};
@@ -755,6 +827,7 @@ int fwd_bwd(Ctx& c, const float* images, const long long* expected, float* loss_
     TCK(cudaMemcpy2DAsync(tp.dlogits, (size_t)VP * 4, dd, (size_t)V * 4, (size_t)V * 4, Md, cudaMemcpyDeviceToDevice, c.st));
     if (loss_out) TCK(cudaMemcpyAsync(loss_out, T->scal, 4, cudaMemcpyDefault, c.st));
   }
+  if (T->drop_on()) { launch_counter_add(T->drop_ctr, 1, c.st); TKL(); }   // the next forward pass draws new masks
   tp.ws_mark = T->ws_used;
   }  // forward phase
   if (phase == PH_FWD) return 0;
@@ -782,9 +855,13 @@ int fwd_bwd(Ctx& c, const float* images, const long long* expected, float* loss_
     if (ln_bwd(c, s.ln3, dy, &dpre3)) return 1;
     // pre3 = f1 + w ; f1 = relu(linear1(f0)) ; f0 = relu(linear0(w))
     WALLOC(df1, (size_t)Md * D); WALLOC(df0, (size_t)Md * FF); WALLOC(dw, (size_t)Md * D);
-    launch_act_bwd(dpre3, s.f1, df1, ACT_RELU, (long long)Md * D, c.st); TKL();       // relu'(pre) == (out > 0)
+    // relu'(pre) == (out > 0); with feed-forward dropout the stored out is the dropped activation (> 0 iff kept and
+    // pre > 0), so dropout's M is in the same test and only its scale remains
+    launch_act_bwd(dpre3, s.f1, df1, ACT_RELU, (long long)Md * D, c.st); TKL();
+    if (T->drop_pffn > 0.f) { launch_axpy(df1, df1, 1.0f / (1.0f - T->drop_pffn), (long long)Md * D, 0, c.st); TKL(); }
     if (lin_bwd(c, df1, D, s.f0, Md, FF, Wl.w_f1, Wl.b_f1, true, D, df0, false)) return 1;
     launch_act_bwd(df0, s.f0, df0, ACT_RELU, (long long)Md * FF, c.st); TKL();
+    if (T->drop_pffn > 0.f) { launch_axpy(df0, df0, 1.0f / (1.0f - T->drop_pffn), (long long)Md * FF, 0, c.st); TKL(); }
     {
       const std::string tp = "dec" + std::to_string(l) + ".";
       tap(c, tp + "d_ffn_out", dpre3, (size_t)Md * D); tap(c, tp + "d_linear1", df1, (size_t)Md * D); tap(c, tp + "d_linear0", df0, (size_t)Md * FF);
@@ -796,12 +873,15 @@ int fwd_bwd(Ctx& c, const float* images, const long long* expected, float* loss_
     // pre2 = out_linear(catt) + u
     WALLOC(dcatt, (size_t)Md * D); WALLOC(du, (size_t)Md * D); WALLOC(dq2, (size_t)Md * D); WALLOC(dkv, (size_t)B * S * 2 * D);
     launch_axpy(du, dpre2, 1.f, (long long)Md * D, 0, c.st); TKL();
-    if (lin_bwd(c, dpre2, D, s.catt, Md, D, Wl.w_co, Wl.b_co, true, D, dcatt, false)) return 1;
+    const float* dco;
+    if (drop_bwd(c, dpre2, (long long)Md * D, drop_site(T, 7, l, false, 1), &dco)) return 1;
+    if (lin_bwd(c, dco, D, s.catt, Md, D, Wl.w_co, Wl.b_co, true, D, dcatt, false)) return 1;
     {
       AttnBwdP a{};
       a.q = s.q2; a.k = s.kv; a.v = s.kv + D; a.dout = dcatt; a.dq = dq2; a.dk = dkv; a.dv = dkv + D;
       a.ldq = D; a.ldk = 2 * D; a.ldv = 2 * D; a.ldo = D; a.lddq = D; a.lddk = 2 * D; a.lddv = 2 * D;
       a.Lq = L; a.Lk = S; a.heads = heads; a.HD = HD; a.causal = 0; a.key_mask = nullptr; a.temperature = temp;
+      a.drop = drop_site(T, 6, l, false, 1);
       int rc = launch_attn_bwd(a, B, c.st);
       if (rc) return tfail(h, "attention backward configuration failed (%d)", rc);
       TKL();
@@ -812,12 +892,15 @@ int fwd_bwd(Ctx& c, const float* images, const long long* expected, float* loss_
     // pre1 = out_linear(att) + x
     WALLOC(datt, (size_t)Md * D); WALLOC(dqkv, (size_t)Md * 3 * D); WALLOC(dx, (size_t)Md * D);
     launch_axpy(dx, dpre1, 1.f, (long long)Md * D, 0, c.st); TKL();
-    if (lin_bwd(c, dpre1, D, s.att, Md, D, Wl.w_so, Wl.b_so, true, D, datt, false)) return 1;
+    const float* dso;
+    if (drop_bwd(c, dpre1, (long long)Md * D, drop_site(T, 5, l, false, 1), &dso)) return 1;
+    if (lin_bwd(c, dso, D, s.att, Md, D, Wl.w_so, Wl.b_so, true, D, datt, false)) return 1;
     {
       AttnBwdP a{};
       a.q = s.qkv; a.k = s.qkv + D; a.v = s.qkv + 2 * D; a.dout = datt; a.dq = dqkv; a.dk = dqkv + D; a.dv = dqkv + 2 * D;
       a.ldq = a.ldk = a.ldv = 3 * D; a.ldo = D; a.lddq = a.lddk = a.lddv = 3 * D;
       a.Lq = L; a.Lk = L; a.heads = heads; a.HD = HD; a.causal = 1; a.key_mask = tp.mask; a.temperature = temp;
+      a.drop = drop_site(T, 4, l, false, 1);
       int rc = launch_attn_bwd(a, B, c.st);
       if (rc) return tfail(h, "attention backward configuration failed (%d)", rc);
       TKL();
@@ -825,6 +908,7 @@ int fwd_bwd(Ctx& c, const float* images, const long long* expected, float* loss_
     if (lin_bwd(c, dqkv, 3 * D, s.x_in, Md, D, Wl.w_sqkv, Wl.b_sqkv, true, 3 * D, dx, true)) return 1;
     dy = dx;
   }
+  if (const DropP d = drop_site(T, 3, 0, false, 1); d.step) { launch_dropout(dy, nullptr, dy, (long long)Md * D, d, 0, 0, c.st); TKL(); }
   launch_embed_bwd(tp.text, dy, T->G + T->emb, Md, D, temp, c.st); TKL();
   bucket_done(c, 0);
   // ---- encoder layers ----
@@ -841,14 +925,17 @@ int fwd_bwd(Ctx& c, const float* images, const long long* expected, float* loss_
     WALLOC(d_ln2, (size_t)Me * C);
     launch_scramble(d_scr, d_ln2, B, S, C, 1, c.st); TKL();
     if (ln_bwd(c, s.ln2, d_ln2, &d_pre2)) return 1;
-    launch_axpy(dxin, d_pre2, 1.f, (long long)Me * C, 1, c.st); TKL();  // pre2 = out_linear(att) + x
+    launch_axpy(dxin, d_pre2, 1.f, (long long)Me * C, 1, c.st); TKL();  // pre2 = dropout(out_linear(att)) + x
     WALLOC(d_att, (size_t)Me * C); WALLOC(d_qkv, (size_t)Me * 3 * C); WALLOC(d_ln1, (size_t)Me * C);
-    if (lin_bwd(c, d_pre2, C, s.att, Me, C, Lw.w_o, Lw.b_o, true, C, d_att, false)) return 1;
+    const float* d_o;
+    if (drop_bwd(c, d_pre2, (long long)Me * C, drop_site(T, 2, i, false, 1), &d_o)) return 1;
+    if (lin_bwd(c, d_o, C, s.att, Me, C, Lw.w_o, Lw.b_o, true, C, d_att, false)) return 1;
     {
       AttnBwdP a{};
       a.q = s.qkv; a.k = s.qkv + C; a.v = s.qkv + 2 * C; a.dout = d_att; a.dq = d_qkv; a.dk = d_qkv + C; a.dv = d_qkv + 2 * C;
       a.ldq = a.ldk = a.ldv = 3 * C; a.ldo = C; a.lddq = a.lddk = a.lddv = 3 * C;
       a.Lq = S; a.Lk = S; a.heads = cf.enc_heads; a.HD = C / cf.enc_heads; a.causal = 0; a.key_mask = nullptr; a.temperature = sqrtf((float)C);
+      a.drop = drop_site(T, 1, i, false, 1);
       int rc = launch_attn_bwd(a, B, c.st);
       if (rc) return tfail(h, "attention backward configuration failed (%d)", rc);
       TKL();
@@ -864,6 +951,12 @@ int fwd_bwd(Ctx& c, const float* images, const long long* expected, float* loss_
     float *dg, *dgp, *dh, *dhp, *dmean;
     WALLOC(dtrunk, (size_t)Me * C); WALLOC(dg, (size_t)B * 2 * C); WALLOC(dgp, (size_t)B * 2 * C); WALLOC(dh, (size_t)B * C / 2);
     WALLOC(dhp, (size_t)B * C / 2); WALLOC(dmean, (size_t)B * C);
+    if (const DropP d = drop_site(T, 0, 0, false, 1); d.step) {   // the PE output's dropout, NCHW mask
+      float* dm;
+      WALLOC(dm, (size_t)Me * C);
+      launch_dropout(de, nullptr, dm, (long long)Me * C, d, S, C, c.st); TKL();
+      de = dm;
+    }
     launch_axpy(dtrunk, de, 1.f, (long long)Me * C, 0, c.st); TKL();
     launch_pe2d_bwd_gate(de, peh, pew, dg, B, tp.H, tp.W, C, c.st); TKL();
     launch_act_bwd(dg, tp.pe_gp, dgp, ACT_SIGMOID, (long long)B * 2 * C, c.st); TKL();
@@ -938,6 +1031,14 @@ int fwd_bwd(Ctx& c, const float* images, const long long* expected, float* loss_
 
 TrainState* state_of(frx_handle* h) { return reinterpret_cast<TrainState*>(h->train); }
 
+// before a forward pass: the device step counter only moves in passes with dropout, so passes without it are counted on
+// the host and added before the next pass with it
+int drop_count_pass(frx_handle* h, TrainState* T, cudaStream_t st) {
+  if (!T->drop_on()) { ++T->drop_pending; return 0; }
+  if (T->drop_pending) { launch_counter_add(T->drop_ctr, T->drop_pending, st); TKL(); T->drop_pending = 0; }
+  return 0;
+}
+
 }  // namespace
 
 // =====================================================================================================================
@@ -966,6 +1067,7 @@ extern "C" int frx_train_create(frx_handle* h, int32_t max_batch, int32_t max_le
   TCK(cudaMalloc(&T->scal, 64)); TCK(cudaMalloc(&T->ones, 4096 * 4)); TCK(cudaMalloc(&T->zeros, 4096 * 4));
   TCK(cudaMemset(T->zeros, 0, 4096 * 4));
   TCK(cudaMalloc(&T->splitk_ws, kSplitKFloats * 4));
+  TCK(cudaMalloc(&T->drop_ctr, sizeof(uint32_t))); TCK(cudaMemset(T->drop_ctr, 0, sizeof(uint32_t)));
   launch_fill(T->ones, 1.f, 4096, 0);
   TCK(cudaDeviceSynchronize());
   // activation tape: ~75 MB (forward) + ~150 MB (backward) of fp32 per image at 128 x 256, plus the decoder's
@@ -993,6 +1095,7 @@ extern "C" void frx_train_destroy(frx_handle* h) {
   TrainState* T = state_of(h);
   cudaFree(T->P); if (T->own_G) cudaFree(T->G); cudaFree(T->M); cudaFree(T->V); cudaFree(T->RS); cudaFree(T->acc); cudaFree(T->sumsq);
   cudaFree(T->scal); cudaFree(T->ones); cudaFree(T->zeros); cudaFree(T->splitk_ws); cudaFree(T->ws); cudaFree(T->img_stage); cudaFree(T->exp_stage);
+  cudaFree(T->drop_ctr);
   for (auto& kv : T->graphs) if (kv.second.exec) cudaGraphExecDestroy(kv.second.exec);
   delete T;
   h->train = nullptr;
@@ -1007,9 +1110,11 @@ extern "C" int frx_train_fwd_bwd(frx_handle* h, const float* images, const int64
   if (B <= 0 || B > T->max_B || L <= 0 || L > T->max_L) return tfail(h, "train_fwd_bwd: batch %d / length %d outside (%d, %d)", B, L, T->max_B, T->max_L);
   DevGuard g; g.enter(h->cfg.device);
   cudaStream_t st = (cudaStream_t)stream;
+  if (drop_count_pass(h, T, st)) return 1;
   // Eager when graphs are off, when a bucket callback wants to start all-reduces between the kernels of the pass, and on
   // the first use of a shape (which also performs the one-time per-device kernel attribute set-up).
-  TrainState::GraphEntry& ge = T->graphs[{B, 2 * L + (h->opt_train_splitk ? 1 : 0)}];   // the launch plan is part of the key
+  // the launch plan and whether dropout runs are part of the key
+  TrainState::GraphEntry& ge = T->graphs[{B, 4 * L + (T->drop_on() ? 2 : 0) + (h->opt_train_splitk ? 1 : 0)}];
   if (!h->opt_graphs || T->bucket_cb || ge.seen++ == 0) {
     Ctx c{h, T, st, B, L};
     return fwd_bwd(c, images, (const long long*)expected, loss_out);
@@ -1060,6 +1165,7 @@ extern "C" int frx_train_forward(frx_handle* h, const float* images, const int64
   const int L = len_plus_1 - 1;
   if (B <= 0 || B > T->max_B || L <= 0 || L > T->max_L) return tfail(h, "train_forward: batch %d / length %d outside (%d, %d)", B, L, T->max_B, T->max_L);
   DevGuard g; g.enter(h->cfg.device);
+  if (drop_count_pass(h, T, (cudaStream_t)stream)) return 1;
   Ctx c{h, T, (cudaStream_t)stream, B, L};
   return fwd_bwd(c, images, (const long long*)expected, loss_out, PH_FWD, logits_out, nullptr);
 }
@@ -1072,6 +1178,49 @@ extern "C" int frx_train_backward(frx_handle* h, const float* images, const floa
   DevGuard g; g.enter(h->cfg.device);
   Ctx c{h, T, (cudaStream_t)stream, B, len_plus_1 - 1};
   return fwd_bwd(c, images, nullptr, nullptr, PH_BWD, nullptr, dlogits);
+}
+
+extern "C" int frx_train_set_dropout(frx_handle* h, float p, float p_ffn, uint64_t seed, int32_t rank) {
+  if (!h) return 1;
+  TrainState* T = state_of(h);
+  if (!T) return tfail(h, "train_set_dropout: call frx_train_create first");
+  if (!(p >= 0.f && p < 1.f) || !(p_ffn >= 0.f && p_ffn < 1.f))
+    return tfail(h, "train_set_dropout: rates must lie in [0, 1) (p = %g, p_ffn = %g)", (double)p, (double)p_ffn);
+  if (rank < 0) return tfail(h, "train_set_dropout: rank %d < 0", (int)rank);
+  if (p == T->drop_p && p_ffn == T->drop_pffn && seed == T->drop_seed && rank == T->drop_rank) return 0;
+  DevGuard g; g.enter(h->cfg.device);
+  // graphs captured with dropout carry the rates and the key as kernel arguments: they go when another setting with
+  // dropout takes over (switching dropout off and on again keeps them)
+  const bool on = p > 0.f || p_ffn > 0.f;
+  if (on && (p != T->graph_p || p_ffn != T->graph_pffn || seed != T->graph_seed || rank != T->graph_rank)) {
+    TCK(cudaDeviceSynchronize());
+    for (auto it = T->graphs.begin(); it != T->graphs.end();) {
+      if (it->first.second & 2) {
+        if (it->second.exec) cudaGraphExecDestroy(it->second.exec);
+        it = T->graphs.erase(it);
+      } else {
+        ++it;
+      }
+    }
+    T->graph_p = p; T->graph_pffn = p_ffn; T->graph_seed = seed; T->graph_rank = rank;
+  }
+  T->drop_p = p; T->drop_pffn = p_ffn; T->drop_seed = seed; T->drop_rank = rank;
+  T->tape.valid = false;   // a frx_train_backward continues a forward pass of the same setting only
+  return 0;
+}
+
+extern "C" int frx_philox4x32(const uint32_t ctr[4], const uint32_t key[2], uint32_t out[4]) {
+  if (!ctr || !key || !out) return 1;
+  uint4 io[2] = {make_uint4(ctr[0], ctr[1], ctr[2], ctr[3]), make_uint4(key[0], key[1], 0, 0)};
+  uint4* d = nullptr;
+  if (cudaMalloc(&d, sizeof io) != cudaSuccess) return 1;
+  bool ok = cudaMemcpy(d, io, sizeof io, cudaMemcpyHostToDevice) == cudaSuccess;
+  if (ok) { launch_philox_probe(d, 0); ok = cudaGetLastError() == cudaSuccess; }
+  ok = ok && cudaMemcpy(io, d, sizeof io, cudaMemcpyDeviceToHost) == cudaSuccess;
+  cudaFree(d);
+  if (!ok) return 1;
+  out[0] = io[0].x; out[1] = io[0].y; out[2] = io[0].z; out[3] = io[0].w;
+  return 0;
 }
 
 extern "C" int frx_train_grad_buffer(frx_handle* h, float** grads, int64_t* count) {

@@ -2,6 +2,8 @@
 #pragma once
 #include <cuda_runtime.h>
 
+#include "common.cuh"
+
 namespace frx {
 
 // dW[n][k] += sum_m dZ[m][n] * A(m, k); A dense [M, lda] or an NHWC activation gathered with the forward geometry
@@ -24,6 +26,7 @@ struct AttnBwdP {
   const unsigned char* key_mask;   // [B][Lk] or nullptr
   float temperature;
   int accumulate_kv;               // dk / dv += instead of =
+  DropP drop;                      // attention dropout of the forward pass (drop.step == nullptr: none)
 };
 
 void launch_fill(float* p, float v, long long n, cudaStream_t st);
@@ -45,7 +48,11 @@ void launch_dw_bwd(const float* dz, const float* x, const float* w, float* dx, f
 void launch_spatial_dot(const float* a, const float* b2, float* out, int B, int S, int C, float scale, cudaStream_t st);
 void launch_spatial_scale(const float* x, const float* g, const float* add, float* out, int B, int S, int C, cudaStream_t st);
 void launch_spatial_add(float* x, const float* add, int B, int S, int C, float scale, cudaStream_t st);
-void launch_pe2d_apply(const float* x, const float* g, const float* peh, const float* pew, float* out, int B, int h, int w, int C, cudaStream_t st);
+void launch_pe2d_apply(const float* x, const float* g, const float* peh, const float* pew, float* out, int B, int h, int w, int C,
+                       const DropP& drop, cudaStream_t st);
+void launch_dropout(const float* x, const float* add, float* y, long long n, const DropP& d, int S, int C, cudaStream_t st);
+void launch_counter_add(uint32_t* ctr, uint32_t v, cudaStream_t st);
+void launch_philox_probe(uint4* io, cudaStream_t st);
 void launch_pe2d_bwd_gate(const float* dout, const float* peh, const float* pew, float* dg, int B, int h, int w, int C, cudaStream_t st);
 void launch_ln_fwd(const float* x, const float* gamma, const float* beta, float* y, float* stat, int M, int C, cudaStream_t st);
 void launch_ln_bwd(const float* dy, const float* x, const float* stat, const float* gamma, float* dx, float* dgamma, float* dbeta, int M, int C,

@@ -257,6 +257,12 @@ def dims_from_flags(FLAGS, num_classes):
         dec_layers=dec.layer_num, dec_heads=dec.head_num, num_classes=num_classes)
 
 
+def dropout_rate_from_flags(FLAGS):
+    """FLAGS.dropout_rate (configs/*.yaml), the rate the reference hands its encoder and decoder; 0 when the flags carry
+    none."""
+    return float(getattr(FLAGS, "dropout_rate", 0.0) or 0.0)
+
+
 class ParamTree(nn.Module):
     """A module that only holds parameters/buffers under reference names."""
 

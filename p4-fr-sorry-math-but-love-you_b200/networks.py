@@ -132,6 +132,8 @@ class _FrxModule(nn.Module):
 
     def _setup(self, FLAGS, train_dataset, precision, max_batch, max_steps):
         self._dims = layout.dims_from_flags(FLAGS, len(train_dataset.id_to_token))
+        self._flags_dropout = layout.dropout_rate_from_flags(FLAGS)
+        self._train_dropout = None   # (p, p_ffn, seed) of set_train_dropout
         t2i = train_dataset.token_to_id
         self._ids = (int(t2i[START]), int(t2i.get(END, 1)), int(t2i[PAD]))
         self._precision = precision
@@ -222,7 +224,8 @@ class EfficientSATRN(_FrxModule):
             # model.train(): BatchNorm batch statistics (and running-statistics updates) like the reference's modules.  The
             # teacher-forced branch (:488-495) is the one the training loop takes (teacher_forcing_ratio 1.0); it returns
             # logits that carry a grad_fn, so criterion(...).backward() fills every parameter's .grad (compatibility path:
-            # parameters / gradients cross the host; EfficientSATRN.train_step is the fused fast path).  Dropout: p = 0.
+            # parameters / gradients cross the host; EfficientSATRN.train_step is the fused fast path).  Dropout: off
+            # unless set_train_dropout enabled it.
             if not (is_train and random.random() < teacher_forcing_ratio):
                 raise NotImplementedError("train mode runs the teacher-forced branch only (teacher_forcing_ratio 1.0, "
                                           "configs/EfficientSATRN.yaml); call .eval() for greedy decoding")
@@ -271,7 +274,37 @@ class EfficientSATRN(_FrxModule):
             eng.h.call("frx_train_create", mb, ml, _ptr(grads))
             tr = eng._train = {"max_batch": mb, "max_len": ml, "grads": grads, "works": [],
                                "scalars": torch.zeros(4, dtype=torch.float32, device=eng.device)}
+            self._apply_train_dropout(eng)
         return eng, tr
+
+    def set_train_dropout(self, p=None, seed=0, p_ffn=0.1):
+        """Train with the reference's dropout (off by default): rate ``p`` (None: FLAGS.dropout_rate) at the 2-D PE
+        output, the attention probabilities and MHA outputs of every encoder / decoder layer and the decoder input;
+        ``p_ffn`` after each decoder feed-forward ReLU (the reference builds Feedforward with its default 0.1 whatever the
+        flag says, EfficientSATRN.py:327, :368-370).  The masks are counter-based (Philox4x32-10 keyed by ``seed``,
+        include/frx.h frx_train_set_dropout), so a run is reproducible; under torch.distributed each rank draws its own.
+        They are not torch's masks.  ``set_train_dropout(0, p_ffn=0)`` turns dropout off again.  Applies to train_step
+        and to the train-mode forward; inference never drops."""
+        p = self._flags_dropout if p is None else float(p)
+        p_ffn = float(p_ffn)
+        for name, r in (("p", p), ("p_ffn", p_ffn)):
+            if not 0.0 <= r < 1.0:
+                raise ValueError("set_train_dropout: %s = %r outside [0, 1)" % (name, r))
+        seed = int(seed)
+        if not 0 <= seed < 1 << 64:
+            raise ValueError("set_train_dropout: seed must fit in 64 unsigned bits")
+        self._train_dropout = (p, p_ffn, seed)
+        eng = self._engine
+        if eng is not None and getattr(eng, "_train", None) is not None:
+            self._apply_train_dropout(eng)
+
+    def _apply_train_dropout(self, eng):
+        if self._train_dropout is None:
+            return
+        import torch.distributed as dist
+        rank = dist.get_rank() if dist.is_available() and dist.is_initialized() else 0
+        p, p_ffn, seed = self._train_dropout
+        eng.h.call("frx_train_set_dropout", p, p_ffn, seed, rank)
 
     def train_step(self, input, expected, lr=5e-4, weight_decay=1e-6, max_grad_norm=2.0, process_group=None,
                    overlap=False, enc_lr=None, dec_lr=None):
